@@ -224,16 +224,17 @@ static_assert(tiles_fit<0>() && tiles_fit<1>() && tiles_fit<2>() && tiles_fit<4>
 // ------------------------------------------------------------------------------------------
 // fused rollout (SURVEY.md 8f item 4, "policy-inference fusion"): T steps in ONE launch, the actions of every step
 // computed in-kernel by a small MLP policy from the observation the previous step left in shared memory
-//   a = tanh(W3 tanh(W2 tanh(W1 obs + b1) + b2) + b3) + sigma * N(0, 1)
-// weights packed input-major: W1[D][H] b1[H] W2[H][H] b2[H] W3[H][8] b3[8], H = 32 or 64.
+//   a = tanh(W3 tanh(W2 tanh(W1 obs + b1) + b2) + b3) + sigma[c] * N(0, 1)
+// weights packed input-major: W1[D][H] b1[H] W2[H][H] b2[H] W3[H][A] b3[A], H = 32 or 64, A = 8 (Ant) or 2 (PointGather).
 // The 4 lanes of an env split the hidden units (H / 4 each); lane k ends up with the two actions of ITS leg.
 // ------------------------------------------------------------------------------------------
 struct RollArgs {
   int T, H;
   const float* w;
-  float sigma;
+  float sigma;            // noise scale of every action component, used when sigma_v is NULL
+  const float* sigma_v;   // [A] per-component noise scale, or NULL
   unsigned long long seed;
-  float* act_out;  // [T][N][8]
+  float* act_out;  // [T][N][A]
 };
 enum { STREAM_POLICY = 6 };
 
@@ -294,8 +295,8 @@ template <int FAMILY, int SUB, int ROLL = 0>
 __global__ void __launch_bounds__(32 * (ROLL ? HRL_ROLL_WARPS : HRL_WARPS_PER_CTA), ROLL ? 2 : Map<SUB>::MIN_CTAS)
 ant_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const float* __restrict__ bounds_g, int n_lines,
                const float* __restrict__ actions, const uint8_t* __restrict__ mask, float* __restrict__ obs_out_g,
-               float* __restrict__ rew_out_g, uint8_t* __restrict__ done_out_g, float* __restrict__ info_out,
-               float* __restrict__ term_out, int mode_g, int n_sub, int D, RollArgs ra = RollArgs()) {
+               float* __restrict__ rew_out_g, uint8_t* __restrict__ done_out_g, float* __restrict__ info_out_g,
+               float* __restrict__ term_out_g, int mode_g, int n_sub, int D, RollArgs ra = RollArgs()) {
   extern __shared__ __align__(16) float smem[];
   typedef Map<SUB> M;
   constexpr int LPE = M::LPE, EPW = M::EPW, IPL = M::IPL;
@@ -369,6 +370,8 @@ ant_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const float*
   float* __restrict__ obs_out = ROLL ? obs_out_g + (size_t)(step + 1) * N * D : obs_out_g;
   float* __restrict__ rew_out = ROLL ? rew_out_g + (size_t)max(step, 0) * N : rew_out_g;
   uint8_t* __restrict__ done_out = ROLL ? done_out_g + (size_t)max(step, 0) * N : done_out_g;
+  float* __restrict__ info_out = ROLL && info_out_g ? info_out_g + (size_t)max(step, 0) * N * 4 : info_out_g;
+  float* __restrict__ term_out = ROLL && term_out_g ? term_out_g + (size_t)max(step, 0) * N * D : term_out_g;
   const float* __restrict__ bounds = bounds_g;
   // ---- physics ----
   float act1 = 0.f, act2 = 0.f;
@@ -388,13 +391,14 @@ ant_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const float*
     if (ROLL) {  // the policy reads the observation the previous pass staged in shared memory (sobs is dense: [EPW][D])
       float* scr = cands + es * 128;
       a = ra.H == 64 ? mlp_policy<16>(wsm, D, sobs + es * D, scr, k) : mlp_policy<8>(wsm, D, sobs + es * D, scr, k);
-      if (ra.sigma > 0.f) {  // exploration noise: Box-Muller on the counter RNG, keyed by (seed, env), addressed by the env's step count
+      if (ra.sigma_v || ra.sigma > 0.f) {  // exploration noise: Box-Muller on the counter RNG, keyed by (seed, env), addressed by the env's step count
+        const float s1 = ra.sigma_v ? __ldg(ra.sigma_v + 2 * k) : ra.sigma, s2 = ra.sigma_v ? __ldg(ra.sigma_v + 2 * k + 1) : ra.sigma;
         float u[4];
         rng_u4(ra.seed, genv, STREAM_POLICY, (uint32_t)T.steps_total, (uint32_t)k, u);
         const float r0 = sqrtf(-2.f * logf(u[0] + 2.98e-8f));
         float sn, cs;
         sincosf(6.2831853f * u[1], &sn, &cs);
-        a.x += ra.sigma * r0 * cs; a.y += ra.sigma * r0 * sn;
+        a.x += s1 * r0 * cs; a.y += s2 * r0 * sn;
       }
       if (active && sub == 0) reinterpret_cast<float2*>(ra.act_out)[((size_t)step * N + e) * 4 + k] = a;
     } else {
@@ -952,18 +956,84 @@ __device__ __forceinline__ void point_substep(V3& pos, V3& vel, V3 force, const 
 }
 
 #define HRL_POINT_EPB 8  // envs per 128-thread block
+#define HRL_POINT_OBS (8 + 2 * HRL_MAX_BINS)  // widest PointGather observation
+
+// PointGather rollout policy: the 16 lanes of an env split the hidden units, lane j owns units U j .. U j + U - 1
+// (U = H / 16: one float4 or float2 of every weight row, the 16 lanes read 256 / 128 contiguous bytes, the 2 envs of a
+// warp read the same addresses: broadcast).  Weights as in mlp_policy, with W3[H][2] b3[2].
+template <int U>
+__device__ __forceinline__ void mlp_layer16(const float* __restrict__ w, const float* __restrict__ b, int n_in, const float* __restrict__ x,
+                                            int j, float (&acc)[U]) {
+  constexpr int H = 16 * U;
+#pragma unroll
+  for (int u = 0; u < U; u++) acc[u] = b[U * j + u];
+#pragma unroll 4
+  for (int i = 0; i < n_in; i++) {
+    const float xi = x[i];
+    const float* wr = w + i * H + U * j;
+    if (U == 4) {
+      const float4 wv = *reinterpret_cast<const float4*>(wr);
+      acc[0] = fmaf(xi, wv.x, acc[0]); acc[1] = fmaf(xi, wv.y, acc[1]); acc[U - 2] = fmaf(xi, wv.z, acc[U - 2]); acc[U - 1] = fmaf(xi, wv.w, acc[U - 1]);
+    } else {
+      const float2 wv = *reinterpret_cast<const float2*>(wr);
+      acc[0] = fmaf(xi, wv.x, acc[0]); acc[U - 1] = fmaf(xi, wv.y, acc[U - 1]);
+    }
+  }
+#pragma unroll
+  for (int u = 0; u < U; u++) acc[u] = tanhf(acc[u]);
+}
+// w: the packed weights in shared memory; obs: this env's staged observation; hid: 64 floats of this env (shared memory)
+template <int U>
+__device__ __forceinline__ float2 mlp_policy16(const float* __restrict__ w, int D, const float* __restrict__ obs, float* __restrict__ hid, int j) {
+  constexpr int H = 16 * U;
+  HRL_CHECK(D <= HRL_POINT_OBS && j >= 0 && j < 16);   // every weight read stays inside the D * H + H + H * H + H + H * 2 + 2 staged floats
+  const float* w1 = w, *b1 = w1 + D * H, *w2 = b1 + H, *b2 = w2 + H * H, *w3 = b2 + H, *b3 = w3 + H * 2;
+  float h[U];
+  mlp_layer16<U>(w1, b1, D, obs, j, h);
+#pragma unroll
+  for (int u = 0; u < U; u++) {
+    HRL_CHECK(U * j + u < 64);
+    hid[U * j + u] = h[u];
+  }
+  __syncwarp();
+  mlp_layer16<U>(w2, b2, H, hid, j, h);
+  __syncwarp();   // hid is rewritten by the next step's first layer
+  float ox = 0.f, oy = 0.f;  // this lane's share of W3 h2, summed over the half-warp
+#pragma unroll
+  for (int u = 0; u < U; u++) {
+    const float2 wv = *reinterpret_cast<const float2*>(w3 + (U * j + u) * 2);
+    ox = fmaf(h[u], wv.x, ox); oy = fmaf(h[u], wv.y, oy);
+  }
+  return make_float2(tanhf(sum16(ox) + b3[0]), tanhf(sum16(oy) + b3[1]));
+}
+#define HRL_POINT_MLP_MAX_FLOATS (HRL_POINT_OBS * 64 + 64 + 64 * 64 + 64 + 64 * 2 + 2)
+
+// ROLL = 1: the fused rollout of PointGather (see ant_env_kernel): step -1 composes the initial observation, steps
+// 0 .. T-1 are full steps whose actions the MLP computes from the observation the previous pass left in sobs; the env
+// state stays in registers in between.  Dynamic shared memory: [EPB][64] hidden activations, then the weights.
+template <int ROLL = 0>
 __global__ void __launch_bounds__(16 * HRL_POINT_EPB)
 point_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const float* __restrict__ actions,
-                 const uint8_t* __restrict__ mask, float* __restrict__ obs_out, float* __restrict__ rew_out,
-                 uint8_t* __restrict__ done_out, float* __restrict__ info_out, float* __restrict__ term_out, int mode,
-                 int n_sub, int D) {
+                 const uint8_t* __restrict__ mask, float* __restrict__ obs_out_g, float* __restrict__ rew_out_g,
+                 uint8_t* __restrict__ done_out_g, float* __restrict__ info_out_g, float* __restrict__ term_out_g, int mode_g,
+                 int n_sub, int D, RollArgs ra = RollArgs()) {
   __shared__ unsigned long long sb[HRL_POINT_EPB][2][HRL_MAX_BINS];
-  __shared__ float sobs[HRL_POINT_EPB][8 + 2 * HRL_MAX_BINS];
+  __shared__ float sobs[HRL_POINT_EPB][HRL_POINT_OBS];
+  extern __shared__ __align__(16) float smem[];
   const int j = threadIdx.x & 15, eb = threadIdx.x >> 4;
   const int e_raw = blockIdx.x * HRL_POINT_EPB + eb;
   const bool valid = e_raw < cfg.num_envs;
+  const int N = cfg.num_envs;
   const int e = valid ? e_raw : cfg.num_envs - 1;  // tail lanes shadow the last env (no stores): every *_sync stays warp-wide
   const uint32_t genv = (uint32_t)(cfg.env_index_offset + e);
+  float* hid = smem + eb * 64;
+  const float* wsm = smem + HRL_POINT_EPB * 64;
+  if (ROLL) {
+    HRL_CHECK(D <= HRL_POINT_OBS && (ra.H == 32 || ra.H == 64));
+    const int nw = D * ra.H + ra.H + ra.H * ra.H + ra.H + ra.H * 2 + 2;
+    for (int i = threadIdx.x; i < nw; i += 16 * HRL_POINT_EPB) const_cast<float*>(wsm)[i] = __ldg(ra.w + i);
+    __syncthreads();
+  }
   const float4 b0 = st.base[e * 4 + 0], b2 = st.base[e * 4 + 2];
   float4 m0 = st.miscf[e * 2 + 0];  // .z running episode return, .w sum of finished returns
   int4 i0 = st.misci[e * 2 + 0];
@@ -972,9 +1042,34 @@ point_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const floa
   const int n_items = cfg.n_food + cfg.n_poison, nb = cfg.n_bins;
   const bool has_item = j < n_items;
   float2 it = reinterpret_cast<const float2*>(st.items)[e * 16 + j];  // item j: food 0..n_food-1, then poison
+#pragma unroll 1
+  for (int step = ROLL ? -1 : 0; step < (ROLL ? ra.T : 1); step++) {
+  const int mode = ROLL ? (step < 0 ? 3 : 0) : mode_g;
+  float* __restrict__ obs_out = ROLL ? obs_out_g + (size_t)(step + 1) * N * D : obs_out_g;
+  float* __restrict__ rew_out = ROLL ? rew_out_g + (size_t)max(step, 0) * N : rew_out_g;
+  uint8_t* __restrict__ done_out = ROLL ? done_out_g + (size_t)max(step, 0) * N : done_out_g;
+  float* __restrict__ info_out = ROLL && info_out_g ? info_out_g + (size_t)max(step, 0) * N * 4 : info_out_g;
+  float* __restrict__ term_out = ROLL && term_out_g ? term_out_g + (size_t)max(step, 0) * N * D : term_out_g;
   if (mode <= 1) {
+    float ax, ay;
+    if (ROLL) {
+      const float2 a = ra.H == 64 ? mlp_policy16<4>(wsm, D, sobs[eb], hid, j) : mlp_policy16<2>(wsm, D, sobs[eb], hid, j);
+      ax = a.x; ay = a.y;
+      if (ra.sigma_v || ra.sigma > 0.f) {  // exploration noise: one Box-Muller pair for the two components (as lane 0 of an ant)
+        const float s1 = ra.sigma_v ? __ldg(ra.sigma_v) : ra.sigma, s2 = ra.sigma_v ? __ldg(ra.sigma_v + 1) : ra.sigma;
+        float u[4];
+        rng_u4(ra.seed, genv, STREAM_POLICY, (uint32_t)i0.z, 0u, u);
+        const float r0 = sqrtf(-2.f * logf(u[0] + 2.98e-8f));
+        float sn, cs;
+        sincosf(6.2831853f * u[1], &sn, &cs);
+        ax += s1 * r0 * cs; ay += s2 * r0 * sn;
+      }
+      if (valid && j == 0) reinterpret_cast<float2*>(ra.act_out)[(size_t)step * N + e] = make_float2(ax, ay);
+    } else {
+      ax = actions[e * 2]; ay = actions[e * 2 + 1];
+    }
     // point_bot.py:28-31: F = a/|a| * 500 N in the world frame (NaN for a == 0: kept, see gather_base.py:99-101)
-    const float ax = actions[e * 2], ay = actions[e * 2 + 1], nn = sqrtf(ax * ax + ay * ay);
+    const float nn = sqrtf(ax * ax + ay * ay);
     const V3 F = mk(ax / nn * cfg.torque_scale, ay / nn * cfg.torque_scale, 0.f), Z = mk(0.f, 0.f, 0.f);
     const SubstepParams P = make_params(cfg);
     const int ns = mode == 0 ? cfg.substeps : n_sub;
@@ -1014,17 +1109,19 @@ point_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const floa
       if (b >= 0) atomicMin(&sb[eb][j < cfg.n_food ? 0 : 1][b], (unsigned long long)__double_as_longlong(d2));
     }
     __syncwarp();
+    // ROLL: sobs of an env without work keeps the observation it emitted last (the policy's next input)
+    const bool compose = !ROLL || work;
     float sa, ca;
     sincosf(atan2f(0.f - pos.y, 0.f - pos.x), &sa, &ca);
     const float o8[8] = {pos.z - initial_z, sa, ca, 0.3f * vel.x, 0.3f * vel.y, 0.3f * vel.z, 0.f, 0.f};
-    if (j < 8) {
+    if (compose && j < 8) {
       float v = o8[0];
 #pragma unroll
       for (int q = 1; q < 8; q++) v = (j == q) ? o8[q] : v;
       sobs[eb][j] = v;
     }
     if (cfg.use_sensor) {
-      for (int b = j; b < 2 * nb; b += 16) {
+      for (int b = j; compose && b < 2 * nb; b += 16) {
         const int ty = b / nb, bb = b - ty * nb;
         const unsigned long long bits = sb[eb][ty][bb];
         sobs[eb][8 + b] = bits == 0x7ff0000000000000ull ? 0.f : (float)(1.0 - __longlong_as_double((long long)bits) / (double)cfg.sensor_range);
@@ -1044,9 +1141,9 @@ point_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const floa
         rank += (same && (od < d2 || (od == d2 && o < j))) ? 1 : 0;
       }
       const int keep_f = min(nb, cfg.n_food), keep_p = min(nb, cfg.n_poison);
-      if (has_item && rank < (poison ? keep_p : keep_f)) {
+      if (compose && has_item && rank < (poison ? keep_p : keep_f)) {
         const int at = 8 + (poison ? 2 * keep_f : 0) + 2 * rank;
-        HRL_CHECK(at >= 0 && at + 1 < 8 + 2 * HRL_MAX_BINS && at + 1 < D);
+        HRL_CHECK(at >= 0 && at + 1 < HRL_POINT_OBS && at + 1 < D);
         sobs[eb][at] = it.x; sobs[eb][at + 1] = it.y;
       }
     }
@@ -1078,6 +1175,7 @@ point_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const floa
     work = again;
     __syncwarp();
   }
+  }  // step loop
   if (valid) {
     if (j == 0) {
       st.base[e * 4 + 0] = make_float4(pos.x, pos.y, pos.z, initial_z);
@@ -1446,7 +1544,7 @@ static int launch_env(hrl_handle* h, int mode, int n_sub, const float* act, cons
   }
   if (h->cfg.env_kind == HRL_POINT_GATHER) {
     const int B = 16 * HRL_POINT_EPB, G = (h->N + HRL_POINT_EPB - 1) / HRL_POINT_EPB;
-    point_env_kernel<<<G, B, 0, s>>>(h->cfg, h->st, act, mask, obs, rew, done, info, term, mode, n_sub, h->D);
+    point_env_kernel<0><<<G, B, 0, s>>>(h->cfg, h->st, act, mask, obs, rew, done, info, term, mode, n_sub, h->D);
   } else {
     const int T = 32 * HRL_WARPS_PER_CTA;
 #define LAUNCH(FAM, SUB)                                                                                                     \
@@ -1601,29 +1699,43 @@ int hrl_flagrun_next_target(hrl_handle* h, const uint8_t* d_mask, void* stream) 
   return HRL_OK;
 }
 
-/* Fused rollout: T env steps in ONE launch with an in-kernel MLP policy (see mlp_policy). */
-int hrl_rollout_mlp(hrl_handle* h, int32_t T, const float* d_weights, int32_t hidden, float sigma, uint64_t noise_seed, float* d_obs,
-                    float* d_act, float* d_rew, uint8_t* d_done, void* stream) {
+/* Fused rollout: T env steps in ONE launch with an in-kernel MLP policy (see mlp_policy / mlp_policy16). */
+int hrl_rollout_mlp_ex(hrl_handle* h, int32_t T, const float* d_weights, int32_t hidden, float sigma, const float* d_sigma,
+                       uint64_t noise_seed, float* d_obs, float* d_act, float* d_rew, uint8_t* d_done, float* d_info,
+                       float* d_terminal_obs, void* stream) {
   if (!h || T < 1 || !d_weights || !d_obs || !d_act || !d_rew || !d_done) return set_err(HRL_E_INVALID, "bad argument to hrl_rollout_mlp");
   if (hidden != 32 && hidden != 64) return set_err(HRL_E_INVALID, "hrl_rollout_mlp: hidden width must be 32 or 64");
-  if (h->cfg.env_kind == HRL_POINT_GATHER) return set_err(HRL_E_INVALID, "hrl_rollout_mlp: Ant envs only");
   if (!(sigma >= 0.f)) return set_err(HRL_E_INVALID, "hrl_rollout_mlp: sigma must be >= 0");
   ON_DEVICE(h->device);
   DevState st = h->st;
   st.fin_flag = nullptr;
   RollArgs ra;
-  ra.T = T; ra.H = hidden; ra.w = d_weights; ra.sigma = sigma; ra.seed = noise_seed; ra.act_out = d_act;
-  const int Tn = 32 * HRL_ROLL_WARPS, EPC = Map<1>::EPW * HRL_ROLL_WARPS, G = (h->N + EPC - 1) / EPC;
-  const int nw = h->D * hidden + hidden + hidden * hidden + hidden + hidden * 8 + 8;
-  const size_t smem = ((size_t)HRL_ROLL_WARPS * Map<1>::SMEM_FLOATS + nw) * sizeof(float);
+  ra.T = T; ra.H = hidden; ra.w = d_weights; ra.sigma = sigma; ra.sigma_v = d_sigma; ra.seed = noise_seed; ra.act_out = d_act;
+  const int nw = h->D * hidden + hidden + hidden * hidden + hidden + hidden * h->A + h->A;
   cudaStream_t s = (cudaStream_t)stream;
-  if (h->cfg.env_kind == HRL_ANT_GATHER)
-    ant_env_kernel<0, 1, 1><<<G, Tn, smem, s>>>(h->cfg, st, h->d_bounds, h->n_lines, nullptr, nullptr, d_obs, d_rew, d_done, nullptr, nullptr, 0, 0, h->D, ra);
-  else
-    ant_env_kernel<1, 1, 1><<<G, Tn, smem, s>>>(h->cfg, st, h->d_bounds, h->n_lines, nullptr, nullptr, d_obs, d_rew, d_done, nullptr, nullptr, 0, 0, h->D, ra);
+  if (h->cfg.env_kind == HRL_POINT_GATHER) {
+    const int G = (h->N + HRL_POINT_EPB - 1) / HRL_POINT_EPB;
+    const size_t smem = ((size_t)HRL_POINT_EPB * 64 + nw) * sizeof(float);
+    point_env_kernel<1><<<G, 16 * HRL_POINT_EPB, smem, s>>>(h->cfg, st, nullptr, nullptr, d_obs, d_rew, d_done, d_info, d_terminal_obs, 0, 0,
+                                                            h->D, ra);
+  } else {
+    const int Tn = 32 * HRL_ROLL_WARPS, EPC = Map<1>::EPW * HRL_ROLL_WARPS, G = (h->N + EPC - 1) / EPC;
+    const size_t smem = ((size_t)HRL_ROLL_WARPS * Map<1>::SMEM_FLOATS + nw) * sizeof(float);
+    if (h->cfg.env_kind == HRL_ANT_GATHER)
+      ant_env_kernel<0, 1, 1><<<G, Tn, smem, s>>>(h->cfg, st, h->d_bounds, h->n_lines, nullptr, nullptr, d_obs, d_rew, d_done, d_info,
+                                                  d_terminal_obs, 0, 0, h->D, ra);
+    else
+      ant_env_kernel<1, 1, 1><<<G, Tn, smem, s>>>(h->cfg, st, h->d_bounds, h->n_lines, nullptr, nullptr, d_obs, d_rew, d_done, d_info,
+                                                  d_terminal_obs, 0, 0, h->D, ra);
+  }
   g_launches++;
   CK(cudaGetLastError());
   return HRL_OK;
+}
+
+int hrl_rollout_mlp(hrl_handle* h, int32_t T, const float* d_weights, int32_t hidden, float sigma, uint64_t noise_seed, float* d_obs,
+                    float* d_act, float* d_rew, uint8_t* d_done, void* stream) {
+  return hrl_rollout_mlp_ex(h, T, d_weights, hidden, sigma, nullptr, noise_seed, d_obs, d_act, d_rew, d_done, nullptr, nullptr, stream);
 }
 
 int hrl_observe(hrl_handle* h, float* d_obs, void* stream) {

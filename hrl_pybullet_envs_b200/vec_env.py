@@ -92,18 +92,37 @@ class HostLazyInfo(LazyInfo):
 class RolloutBuffer:
     """[T, N, ...] CUDA tensors the env kernel writes into directly (SURVEY.md 8f-4: the consumer side keeps the
     observations on the device; a trainer reads obs[t] / rew[t] / done[t] without any copy in between).
-    obs has T + 1 slots: slot 0 takes the reset observation, step t writes obs[t + 1], rew[t], done[t]."""
+    obs has T + 1 slots: slot 0 takes the reset observation, step t writes obs[t + 1], rew[t], done[t].
+    With ``info=True`` it also holds info[T, N, 4] (the four columns of ``step()``'s info per step), with
+    ``terminal_obs=True`` terminal_obs[T, N, D]: row e of slot t is the observation before the auto-reset of an env that
+    finished in step t (other rows are stale) - what a value bootstrap at a TimeLimit truncation needs."""
 
-    def __init__(self, env, horizon):
+    def __init__(self, env, horizon, info=False, terminal_obs=False):
         d = env.device
         self.T = int(horizon)
+        self.kind = env.kind
         self.obs = torch.zeros(self.T + 1, env.N, env.D, device=d)
         self.act = torch.zeros(self.T, env.N, env.A, device=d)
         self.rew = torch.zeros(self.T, env.N, device=d)
         self.done = torch.zeros(self.T, env.N, dtype=torch.bool, device=d)
+        self.info = torch.zeros(self.T, env.N, 4, device=d) if info else None
+        self.terminal_obs = torch.zeros(self.T, env.N, env.D, device=d) if terminal_obs else None
 
     def slot(self, t):
         return self.obs[t + 1], self.rew[t], self.done[t]
+
+    @property
+    def truncated(self):
+        """bool [T, N]: the episode ended in step t by the TimeLimit, not by the env (``info["TimeLimit.truncated"]``)."""
+        if self.info is None:
+            raise ValueError("this RolloutBuffer holds no info (create it with info=True)")
+        return (self.info[..., 2] % 2) > 0
+
+    def infos(self, t):
+        """``info`` of step t, the mapping ``step()`` returns (with "terminal_obs" when the buffer holds them)."""
+        if self.info is None:
+            raise ValueError("this RolloutBuffer holds no info (create it with info=True)")
+        return LazyInfo(self.info[t], self.kind, None if self.terminal_obs is None else self.terminal_obs[t])
 
 
 class VecEnv:
@@ -201,7 +220,8 @@ class VecEnv:
     def step(self, actions, want_terminal_obs=False, out=None):
         """actions: float32 CUDA tensor [N, A] (device path) or numpy array (host path).
         ``out=(obs[N, D] f32, rew[N] f32, done[N] u8/bool)``: the kernel writes this step's results straight into
-        those CUDA tensors (e.g. slot t of a ``RolloutBuffer``) instead of the env's own buffers - no copy."""
+        those CUDA tensors (e.g. slot t of a ``RolloutBuffer``) instead of the env's own buffers - no copy.  A fourth
+        tensor ``info[N, 4] f32`` takes the raw info columns the same way."""
         if isinstance(actions, np.ndarray):
             return self.step_host(actions)
         a = actions
@@ -214,26 +234,30 @@ class VecEnv:
             if self._term is None:
                 self._term = torch.zeros(self.N, self.D, device=self.device)
             term = self._term
-        obs, rew, done = self._obs, self._rew, self._done
+        obs, rew, done, info = self._obs, self._rew, self._done, self._info
         if out is not None:
-            obs, rew, done = out
+            if len(out) not in (3, 4):
+                raise ValueError("out must be (obs, rew, done) or (obs, rew, done, info)")
+            obs, rew, done = out[:3]
+            info = out[3] if len(out) == 4 else info
             for t, shape, dts in ((obs, (self.N, self.D), (torch.float32,)), (rew, (self.N,), (torch.float32,)),
-                                  (done, (self.N,), (torch.uint8, torch.bool))):
+                                  (done, (self.N,), (torch.uint8, torch.bool)), (info, (self.N, 4), (torch.float32,))):
                 if tuple(t.shape) != shape or t.dtype not in dts or not t.is_contiguous() or t.device != self.device:
                     raise ValueError("out tensors must be contiguous CUDA tensors obs[%d,%d] f32, rew[%d] f32, done[%d] u8/bool"
-                                     % (self.N, self.D, self.N, self.N))
+                                     ", info[%d,4] f32" % (self.N, self.D, self.N, self.N, self.N))
         if _NVTX:
             torch.cuda.nvtx.range_push("hrl.step")
         _cabi.check(self.L.hrl_step(self.h, _ptr(a), _ptr(obs), _ptr(rew), _ptr(done),
-                                    _ptr(self._info), _ptr(term), self._stream()))
+                                    _ptr(info), _ptr(term), self._stream()))
         if _NVTX:
             torch.cuda.nvtx.range_pop()
-        return obs, rew, done.view(torch.bool), self._info_dict(self._info, term)
+        return obs, rew, done.view(torch.bool), self._info_dict(info, term)
 
     def capture_rollout(self, actions, buf=None):
         """CUDA-graph launch (SURVEY.md section 7 step 5): capture ``T = actions.shape[0]`` consecutive steps, step t
         reading ``actions[t]`` (a [T, N, A] CUDA tensor the caller refills between replays) and writing slot t of
-        ``buf`` (a ``RolloutBuffer``; created when None).  Returns ``(graph, buf)``; ``graph.replay()`` runs the T
+        ``buf`` (a ``RolloutBuffer``; created when None), its ``info[t]`` too when the buffer holds info (terminal
+        observations are not recorded here).  Returns ``(graph, buf)``; ``graph.replay()`` runs the T
         steps with ONE launch from the host.  ``step()`` itself is capture-safe (no allocation, no synchronisation),
         so a caller can equally capture its own policy + ``env.step`` loop with ``torch.cuda.graph``."""
         a = actions
@@ -247,7 +271,7 @@ class VecEnv:
         g = torch.cuda.CUDAGraph()
         with torch.cuda.graph(g):
             for t in range(T):
-                self.step(a[t], out=buf.slot(t))
+                self.step(a[t], out=buf.slot(t) if buf.info is None else buf.slot(t) + (buf.info[t],))
         return g, buf
 
     @staticmethod
@@ -259,27 +283,40 @@ class VecEnv:
             parts += [W.detach().to(torch.float32).t().contiguous().reshape(-1), b.detach().to(torch.float32).reshape(-1)]
         return torch.cat(parts).contiguous()
 
-    def rollout_mlp(self, layers, horizon, buf=None, sigma=0.0, noise_seed=0):
-        """Fused rollout (include/hrl_b200.h `hrl_rollout_mlp`): `horizon` steps in ONE kernel launch, actions from the
-        3-layer tanh MLP `layers` = ((W1[H, D], b1), (W2[H, H], b2), (W3[8, H], b3)) evaluated inside the kernel (H = 32 or
-        64), plus N(0, sigma^2) exploration noise.  Fills and returns a RolloutBuffer: obs[0..T], act, rew, done."""
-        if self.kind == HRL_POINT_GATHER:
-            raise TypeError("rollout_mlp: Ant envs only")
+    def rollout_mlp(self, layers, horizon, buf=None, sigma=0.0, noise_seed=0, want_info=False, want_terminal_obs=False):
+        """Fused rollout (include/hrl_b200.h `hrl_rollout_mlp_ex`): `horizon` steps in ONE kernel launch, actions from the
+        3-layer tanh MLP `layers` = ((W1[H, D], b1), (W2[H, H], b2), (W3[A, H], b3)) evaluated inside the kernel (H = 32 or
+        64), plus N(0, sigma^2) exploration noise.  `sigma` is a float or a length-A tensor (one scale per action
+        component, e.g. exp(log_std) of a Gaussian policy).  Fills and returns a RolloutBuffer: obs[0..T], act, rew,
+        done, and with `want_info` / `want_terminal_obs` also info / terminal_obs (allocated when `buf` is None)."""
         (W1, b1), (W2, b2), (W3, b3) = layers
         H = W1.shape[0]
         if H not in (32, 64) or tuple(W1.shape) != (H, self.D) or tuple(W2.shape) != (H, H) or tuple(W3.shape) != (self.A, H):
             raise ValueError("layers must be ((W1[H,%d], b1[H]), (W2[H,H], b2[H]), (W3[%d,H], b3[%d])) with H = 32 or 64" % (self.D, self.A, self.A))
         w = self.pack_mlp(layers).to(self.device)
-        buf = buf or RolloutBuffer(self, horizon)
+        sig_v = None
+        if isinstance(sigma, torch.Tensor):
+            sig_v = sigma.detach().to(device=self.device, dtype=torch.float32).contiguous()
+            if tuple(sig_v.shape) != (self.A,):
+                raise ValueError("sigma must be a float or a tensor of %d entries, got shape %s" % (self.A, tuple(sig_v.shape)))
+            if not bool((torch.isfinite(sig_v) & (sig_v >= 0)).all()):
+                raise ValueError("sigma entries must be finite and >= 0")
+            sigma = 0.0
+        buf = buf or RolloutBuffer(self, horizon, info=want_info, terminal_obs=want_terminal_obs)
         if buf.T < horizon:
             raise ValueError("rollout buffer holds %d steps, need %d" % (buf.T, horizon))
+        if (want_info and buf.info is None) or (want_terminal_obs and buf.terminal_obs is None):
+            raise ValueError("rollout buffer has no room for info / terminal_obs: create it with info=True / terminal_obs=True")
+        info = buf.info if want_info else None
+        term = buf.terminal_obs if want_terminal_obs else None
         if _NVTX:
             torch.cuda.nvtx.range_push("hrl.rollout_mlp")
-        _cabi.check(self.L.hrl_rollout_mlp(self.h, int(horizon), _ptr(w), int(H), float(sigma), int(noise_seed), _ptr(buf.obs), _ptr(buf.act),
-                                           _ptr(buf.rew), _ptr(buf.done), self._stream()))
+        _cabi.check(self.L.hrl_rollout_mlp_ex(self.h, int(horizon), _ptr(w), int(H), float(sigma), _ptr(sig_v), int(noise_seed),
+                                              _ptr(buf.obs), _ptr(buf.act), _ptr(buf.rew), _ptr(buf.done), _ptr(info), _ptr(term),
+                                              self._stream()))
         if _NVTX:
             torch.cuda.nvtx.range_pop()
-        self._keep = w   # the launch is asynchronous: keep the packed weights alive
+        self._keep = (w, sig_v)   # the launch is asynchronous: keep the packed weights and noise scales alive
         return buf
 
     def rollout_buffer(self, horizon):

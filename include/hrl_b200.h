@@ -211,6 +211,21 @@ int hrl_host_layout(const hrl_config* cfg, size_t* off_rew, size_t* off_info, si
 int hrl_rollout_mlp(hrl_handle* h, int32_t T, const float* d_weights, int32_t hidden, float sigma, uint64_t noise_seed,
                     float* d_obs, float* d_act, float* d_rew, uint8_t* d_done, void* stream);
 
+/* hrl_rollout_mlp for training (hrl_rollout_mlp is this call with d_sigma, d_info and d_terminal_obs NULL).  Every env
+ * family, PointGather included (act_dim A = 2: W3[H][2] b3[2]; Ant: A = 8).  The buffers a trainer needs besides those above:
+ *   d_sigma        f32[A] or NULL: action component c gets noise d_sigma[c] * N(0, 1) (the same draw as for the scalar
+ *                  sigma, so d_sigma filled with s gives the actions of sigma = s); entries must be finite and >= 0, which
+ *                  the caller checks (reading them here would cost a synchronisation).  NULL: the scalar sigma for all.
+ *   d_info         f32[T, N, 4] or NULL: slot t holds what hrl_step writes to d_info for step t (bit 0 of column 2 tells a
+ *                  TimeLimit truncation from a termination).
+ *   d_terminal_obs f32[T, N, obs_dim] or NULL: row e of slot t is written only when env e finished in step t, with its
+ *                  observation from before the auto-reset (d_obs[t + 1] already holds the reset observation); other rows
+ *                  are left untouched, as in hrl_step.
+ * d_act f32[T, N, A]; T >= 1; hidden = 32 or 64. */
+int hrl_rollout_mlp_ex(hrl_handle* h, int32_t T, const float* d_weights, int32_t hidden, float sigma, const float* d_sigma,
+                       uint64_t noise_seed, float* d_obs, float* d_act, float* d_rew, uint8_t* d_done, float* d_info,
+                       float* d_terminal_obs, void* stream);
+
 /* Replaces saveState/restoreState (used as the reset mechanism by pybullet_envs) and gives
  * the "identical saved states" hook the one-step parity tests need.
  *   d_fstate f32[N, HRL_STATE_F], d_istate i32[N, HRL_STATE_I]. */
