@@ -25,7 +25,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
 
 # every symbol include/hrl_b200.h declares (checked by tests/test_cabi_symbols.py)
 SYMBOLS = ["hrl_default_config", "hrl_obs_dim", "hrl_act_dim", "hrl_create", "hrl_destroy", "hrl_reset", "hrl_step",
-           "hrl_step_host", "hrl_set_host_mode", "hrl_host_layout", "hrl_get_state", "hrl_set_state", "hrl_observe", "hrl_gather_sensor", "hrl_sense_walls",
+           "hrl_step_host", "hrl_set_host_mode", "hrl_host_layout", "hrl_get_state", "hrl_set_state", "hrl_observe", "hrl_gather_sensor", "hrl_sense_walls", "hrl_gae",
            "hrl_substeps", "hrl_rollout_mlp", "hrl_rollout_mlp_ex", "hrl_flagrun_next_target", "hrl_get_stats", "hrl_stream_gate", "hrl_set_lanes_per_env", "hrl_get_lanes_per_env", "hrl_launch_count", "hrl_last_error", "hrl_version"]
 
 
@@ -77,6 +77,7 @@ def lib():
     L.hrl_observe.argtypes = [vp, vp, vp]
     L.hrl_gather_sensor.argtypes = [i32, i32, f32, f32, vp, vp, vp, vp, vp, vp, vp]
     L.hrl_sense_walls.argtypes = [i32, i32, f32, f32, i32, vp, vp, vp, vp, vp]
+    L.hrl_gae.argtypes = [i32, i32, f32, f32] + [vp] * 8
     L.hrl_substeps.argtypes = [vp, vp, i32, vp]
     L.hrl_rollout_mlp.argtypes = [vp, i32, vp, i32, f32, C.c_uint64, vp, vp, vp, vp, vp]
     L.hrl_rollout_mlp_ex.argtypes = [vp, i32, vp, i32, f32, vp, C.c_uint64, vp, vp, vp, vp, vp, vp, vp]

@@ -18,6 +18,7 @@
 #include "../../include/hrl_b200.h"
 #include "hrl_ant.cuh"
 #include "hrl_ant_wide.cuh"
+#include "hrl_gae.cuh"
 #include "hrl_math.cuh"
 #include "hrl_sensors.cuh"
 
@@ -1785,6 +1786,25 @@ int hrl_sense_walls(int32_t M, int32_t n_bins, float span, float range, int32_t 
   if (M == 0) return HRL_OK;
   const int T = 128, G = (M * n_bins + T - 1) / T;
   sense_walls_kernel<<<G, T, 0, (cudaStream_t)stream>>>(M, n_bins, span, range, n_lines, d_bounds, d_xy, d_yaw, d_out);
+  g_launches++;
+  CK(cudaGetLastError());
+  return HRL_OK;
+}
+
+/* GAE(lambda) over a rollout buffer (gae_kernel, hrl_gae.cuh); runs on the current device. */
+int hrl_gae(int32_t T, int32_t N, float gamma, float lam, const float* d_rew, const uint8_t* d_done, const float* d_info,
+            const float* d_values, const float* d_terminal_values, float* d_adv, float* d_ret, void* stream) {
+  if (T < 1 || N < 1 || !d_rew || !d_done || !d_values || !d_adv) return set_err(HRL_E_INVALID, "bad argument to hrl_gae");
+  if (!(gamma >= 0.f && gamma <= 1.f) || !(lam >= 0.f && lam <= 1.f))
+    return set_err(HRL_E_INVALID, "hrl_gae: gamma and lam must lie in [0, 1]");
+  if (!d_info != !d_terminal_values)
+    return set_err(HRL_E_INVALID, "hrl_gae: d_info and d_terminal_values must both be given or both be NULL");
+  int dev = 0, sms = 0;
+  CK(cudaGetDevice(&dev));
+  CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  const int W = gae_warps(T, N, sms), L = (T + W - 1) / W;
+  gae_kernel<<<(N + 31) / 32, 32 * W, 0, (cudaStream_t)stream>>>(T, N, L, gamma, gamma * lam, d_rew, d_done, d_info, d_values,
+                                                                 d_terminal_values, d_adv, d_ret);
   g_launches++;
   CK(cudaGetLastError());
   return HRL_OK;

@@ -124,6 +124,45 @@ class RolloutBuffer:
             raise ValueError("this RolloutBuffer holds no info (create it with info=True)")
         return LazyInfo(self.info[t], self.kind, None if self.terminal_obs is None else self.terminal_obs[t])
 
+    def gae(self, values, gamma=0.99, lam=0.95, terminal_values=None, out=None):
+        """GAE(lambda) advantages and returns of the T steps in this buffer, in ONE kernel launch (include/hrl_b200.h
+        `hrl_gae`).  ``values``: float32 [T + 1, N], V(obs[0..T]).  ``terminal_values``: float32 [T, N], typically
+        ``critic(buf.terminal_obs)`` over the whole tensor (stale rows included: a row is read only where it is selected);
+        it needs a buffer made with ``info=True``.  With it, an episode ended by the TimeLimit bootstraps from
+        ``terminal_values[t]`` and one ended by the env from 0; without it, every done is a termination.  ``obs[t + 1]`` of
+        an env that finished in step t is the reset observation, so its value never bootstraps step t.
+        ``out=(adv, ret)``: float32 [T, N] tensors written in place (no allocation, so the call can be captured in a CUDA
+        graph).  No host synchronisation.  Returns ``(adv, ret)``."""
+        T, N = self.rew.shape
+        dev = self.rew.device
+
+        def check(name, t, shape):
+            if not isinstance(t, torch.Tensor) or tuple(t.shape) != shape or t.dtype != torch.float32 or not t.is_contiguous() \
+                    or t.device != dev:
+                raise ValueError("%s must be a contiguous float32 tensor [%s] on %s" % (name, ", ".join(map(str, shape)), dev))
+
+        check("values", values, (T + 1, N))
+        if terminal_values is not None:
+            if self.info is None:
+                raise ValueError("terminal_values need the truncation flags: create the RolloutBuffer with info=True")
+            check("terminal_values", terminal_values, (T, N))
+        if not (0.0 <= gamma <= 1.0 and 0.0 <= lam <= 1.0):
+            raise ValueError("gamma and lam must lie in [0, 1], got %r, %r" % (gamma, lam))
+        if out is None:
+            adv, ret = torch.empty_like(self.rew), torch.empty_like(self.rew)
+        else:
+            if len(out) != 2:
+                raise ValueError("out must be (adv, ret)")
+            adv, ret = out
+            check("out[0] (adv)", adv, (T, N))
+            check("out[1] (ret)", ret, (T, N))
+        info = self.info if terminal_values is not None else None
+        with torch.cuda.device(dev):
+            _cabi.check(_cabi.lib().hrl_gae(T, N, float(gamma), float(lam), _ptr(self.rew), _ptr(self.done), _ptr(info), _ptr(values),
+                                            _ptr(terminal_values), _ptr(adv), _ptr(ret),
+                                            C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
+        return adv, ret
+
 
 class VecEnv:
     """N independent envs of one reference id on one GPU.

@@ -251,6 +251,19 @@ int hrl_gather_sensor(int32_t M, int32_t n_bins, float sensor_range, float senso
 /* Wall lidar, sizeable_enclosed_scene.py:63-97.  d_bounds f32[n_lines,4] (x1,y1,x2,y2). */
 int hrl_sense_walls(int32_t M, int32_t n_bins, float span, float range, int32_t n_lines,
                     const float* d_bounds, const float* d_xy, const float* d_yaw, float* d_out, void* stream);
+/* GAE(lambda) over a rollout buffer (no counterpart in the reference; DESIGN.md section 4, kernel 7).  Stateless, no handle;
+ * runs on the current device.  ONE launch, no atomics: the same inputs give the same bytes on every call.
+ *   d_rew f32[T,N], d_done u8[T,N], d_values f32[T+1,N] (V of obs[0..T]),
+ *   d_info f32[T,N,4] and d_terminal_values f32[T,N]: both NULL (every done terminates) or both non-NULL,
+ *   d_adv f32[T,N], d_ret f32[T,N] or NULL.  0 <= gamma, lam <= 1.  Asynchronous on `stream`, no host synchronisation.
+ * For env e and step t:
+ *   next_t  = d_terminal_values[t,e] if done and bit 0 (TimeLimit truncation) of int(d_info[t,e,2]) is set,
+ *             0 if done otherwise (bit 1, the Flagrun goal switch, is ignored), d_values[t+1,e] if not done;
+ *   delta_t = rew + gamma next_t - values[t,e];  A_t = delta_t + gamma lam (1 - done_t) A_{t+1}, A_T = 0;  ret_t = A_t + values[t,e].
+ * Values that are not selected are never operands: stale terminal-value rows and the value after a termination may hold
+ * anything, NaN included.  d_adv / d_ret must not overlap the inputs. */
+int hrl_gae(int32_t T, int32_t N, float gamma, float lam, const float* d_rew, const uint8_t* d_done, const float* d_info,
+            const float* d_values, const float* d_terminal_values, float* d_adv, float* d_ret, void* stream);
 /* `n_sub` physics sub-steps on the handle's current state (no task logic, no reset):
  * replaces scene.global_step() -> p.stepSimulation() (ant_gather_env.py:78). */
 int hrl_substeps(hrl_handle* h, const float* d_actions, int32_t n_sub, void* stream);
