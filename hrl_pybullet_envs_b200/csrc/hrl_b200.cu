@@ -1436,6 +1436,16 @@ int hrl_set_lanes_per_env(hrl_handle* h, int32_t lanes) {
 }
 int hrl_get_lanes_per_env(const hrl_handle* h) { return h ? 4 * h->sub : -1; }
 
+int hrl_set_compact_rows(hrl_handle* h, int32_t on) {
+  if (!h) return set_err(HRL_E_INVALID, "null handle");
+  h->compact = on != 0;
+  return HRL_OK;
+}
+// what launch_env runs: the compact rows exist only in the 4-lane Ant kernel
+int hrl_get_compact_rows(const hrl_handle* h) {
+  return h ? (h->cfg.env_kind != HRL_POINT_GATHER && h->sub == 1 && h->compact) : -1;
+}
+
 int hrl_destroy(hrl_handle* h) {
   if (!h) return HRL_OK;
   DeviceGuard guard(h->device);

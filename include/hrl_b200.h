@@ -273,6 +273,15 @@ int hrl_substeps(hrl_handle* h, const float* d_actions, int32_t n_sub, void* str
  * New handles take the library default, or HRL_B200_LANES from the environment.  DESIGN.md section 4. */
 int hrl_set_lanes_per_env(hrl_handle* h, int32_t lanes);
 int hrl_get_lanes_per_env(const hrl_handle* h);
+/* Solver-row layout of the 4-lane Ant kernel: 14-wide rows, or compact rows (the 8 non-zeros of a row + its leg index,
+ * expanded to 14 wide on load; smaller shared memory, so 7 CTAs per SM instead of 6).  Results agree up to float32
+ * rounding: the compiler contracts a few multiply-adds differently in the two kernels.
+ * hrl_create picks compact when it saves a whole wave of CTAs at the device's SM count; HRL_B200_COMPACT=0|1 in the
+ * environment overrides that for new handles.  set: any handle (HRL_E_INVALID for NULL).  get: 1 iff the next step,
+ * reset, observe or substeps launch uses the compact rows (an Ant env with 4 lanes per env and the flag set), 0 if not,
+ * -1 for NULL.  The fused rollout (hrl_rollout_mlp*) always uses the 14-wide rows. */
+int hrl_set_compact_rows(hrl_handle* h, int32_t on);
+int hrl_get_compact_rows(const hrl_handle* h);
 
 /* In-kernel counters feeding the FLOP model of bench.py (SURVEY.md section 5 "in-kernel optional counters"):
  * out = {contacts, joint-limit rows, env-substeps, reserved} accumulated since the last reset; synchronises. */

@@ -1,7 +1,8 @@
 """Workload for the bounds-checked build (-DHRL_BOUNDS=1 -> libhrl_b200_chk.so; run with HRL_B200_LIB pointing at it):
-every env family and lane mapping, ragged batch, short episodes (resets inside the run), saturated actions, and ants
-thrown at walls / dropped upside down so that the contact-slot, row and candidate indices reach their largest values.
-A device-side assert aborts the process.  Used by tests/test_gpu_bounds_build.py (compute-sanitizer is closed on the pool)."""
+every env family and Ant kernel variant (4 lanes per env with 14-wide or compact solver rows, 8 and 16 lanes), ragged
+batch, short episodes (resets inside the run), saturated actions, and ants thrown at walls / dropped upside down so
+that the contact-slot, row and candidate indices reach their largest values.  A device-side assert aborts the process.
+Used by tests/test_gpu_bounds_build.py (compute-sanitizer is closed on the pool)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -15,11 +16,15 @@ CASES = [("AntGatherBulletEnv-v0", {}), ("AntGatherBulletEnv-v0", dict(use_senso
          ("AntFlagrunBulletEnv-v0", dict(max_targets=0, max_target_dist=2.0)), ("AntMjBulletEnv-v0", {}), ("AntMazeMjEnv-v0", {}),
          ("PointGatherBulletEnv-v0", {}), ("PointGatherBulletEnv-v0", dict(use_sensor=False))]
 g = torch.Generator(device="cuda").manual_seed(5)
+# (lanes per env, compact rows): at N = 203 hrl_create picks the 14-wide rows, so the compact ones are forced here
+ANT_VARIANTS = ((4, 0), (4, 1), (8, 0), (16, 0))
 for env_id, kw in CASES:
-    for lanes in ((4, 8, 16) if "Point" not in env_id else (4,)):
+    for lanes, compact in (ANT_VARIANTS if "Point" not in env_id else ((4, 0),)):
         env = VecEnv(env_id, N, seed=1, max_episode_steps=25, **kw)
         if lanes != 4:
             _cabi.check(env.L.hrl_set_lanes_per_env(env.h, lanes))
+        _cabi.check(env.L.hrl_set_compact_rows(env.h, compact))
+        assert env.L.hrl_get_compact_rows(env.h) == (compact if "Point" not in env_id else 0)
         env.reset()
         for t in range(60):
             a = torch.rand(N, env.A, generator=g, device="cuda") * 2 - 1
@@ -42,6 +47,6 @@ for env_id, kw in CASES:
         env.step(np.random.uniform(-1, 1, (N, env.A)).astype(np.float32))   # host path
         env.observe()
         torch.cuda.synchronize()
-        print("ok", env_id, kw, "lanes", lanes)
+        print("ok", env_id, kw, "lanes", lanes, "compact", compact)
         env.close()
 print("bounds run complete")
