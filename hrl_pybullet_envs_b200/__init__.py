@@ -7,13 +7,16 @@
 from .config import ENV_IDS, HrlConfig  # noqa: F401
 from .gym_shim import Box, make, register, registry  # noqa: F401
 
-__all__ = ["ENV_IDS", "HrlConfig", "Box", "make", "register", "registry", "VecEnv", "RolloutBuffer"]
+__all__ = ["ENV_IDS", "HrlConfig", "Box", "make", "register", "registry", "VecEnv", "RolloutBuffer", "RunningNormalizer"]
 
 
 def __getattr__(name):  # torch is only needed for the CUDA path
     if name in ("VecEnv", "RolloutBuffer"):
         from . import vec_env
         return getattr(vec_env, name)
+    if name == "RunningNormalizer":
+        from . import normalize
+        return normalize.RunningNormalizer
     if name in ("gather_sensor", "sense_walls"):
         from . import vec_env
         return getattr(vec_env, name)

@@ -13,13 +13,16 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <atomic>
+#include <utility>
 
 #include "../../include/hrl_b200.h"
 #include "hrl_ant.cuh"
 #include "hrl_ant_wide.cuh"
 #include "hrl_gae.cuh"
 #include "hrl_math.cuh"
+#include "hrl_normalize.cuh"
 #include "hrl_sensors.cuh"
 
 #ifndef HRL_WARPS_PER_CTA
@@ -236,6 +239,10 @@ struct RollArgs {
   const float* sigma_v;   // [A] per-component noise scale, or NULL
   unsigned long long seed;
   float* act_out;  // [T][N][A]
+  // ROLL = 2 only: the policy reads clamp((obs - mean) * rstd, -clip, clip) (hrl_rollout_mlp_norm)
+  const float* obs_mean;  // [D]
+  const float* obs_rstd;  // [D]
+  float obs_clip;
 };
 enum { STREAM_POLICY = 6 };
 
@@ -285,6 +292,11 @@ __device__ __forceinline__ float2 mlp_policy(const float* __restrict__ w, int D,
   __syncwarp();
   return make_float2(tanhf(o.x), tanhf(o.y));
 }
+// Normalized policy input of obs component i: subtract, multiply, clamp, each rounded on its own (no FMA can form), so
+// torch.clamp((obs - mean) * rstd, -clip, clip) gives the same bits.  stat: mean[D] then rstd[D], staged in shared memory.
+__device__ __forceinline__ float norm_obs(float o, const float* __restrict__ stat, int D, int i, float clip) {
+  return fminf(fmaxf(__fmul_rn(__fsub_rn(o, stat[i]), stat[D + i]), -clip), clip);
+}
 #define HRL_ROLL_WARPS 2                       // warps per CTA of the fused-rollout instantiations (they share the weights)
 #define HRL_MLP_MAX_FLOATS (60 * 64 + 64 + 64 * 64 + 64 + 64 * 8 + 8)   // obs_dim <= 60, H <= 64
 
@@ -292,6 +304,7 @@ __device__ __forceinline__ float2 mlp_policy(const float* __restrict__ w, int D,
 __device__ float* g_dbg_contacts = nullptr;  // [N][4 legs][40]: candidate lists of the first sub-step of the last launch
 #endif
 
+// ROLL = 1: the fused rollout; ROLL = 2: the same with a normalized policy input (hrl_rollout_mlp_norm)
 template <int FAMILY, int SUB, int ROLL = 0>
 __global__ void __launch_bounds__(32 * (ROLL ? HRL_ROLL_WARPS : HRL_WARPS_PER_CTA), ROLL ? 2 : Map<SUB>::MIN_CTAS)
 ant_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const float* __restrict__ bounds_g, int n_lines,
@@ -306,9 +319,13 @@ ant_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const float*
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, l = lane & (LPE - 1), k = l & 3, sub = l >> 2, ew = lane / LPE, es = ew;
   float* rows = smem + warp * M::SMEM_FLOATS;
   const float* wsm = smem + WPC * M::SMEM_FLOATS;   // ROLL: the policy weights, behind the warps' own regions
+  // ROLL = 2: the observation statistics (mean[D], rstd[D]) behind the weights
+  const float* nstat = wsm + (ROLL == 2 ? D * ra.H + ra.H + ra.H * ra.H + ra.H + ra.H * 8 + 8 : 0);
   if (ROLL) {
     const int nw = D * ra.H + ra.H + ra.H * ra.H + ra.H + ra.H * 8 + 8;
     for (int i = threadIdx.x; i < nw; i += 32 * WPC) const_cast<float*>(wsm)[i] = __ldg(ra.w + i);
+    if (ROLL == 2)
+      for (int i = threadIdx.x; i < 2 * D; i += 32 * WPC) const_cast<float*>(nstat)[i] = __ldg(i < D ? ra.obs_mean + i : ra.obs_rstd + (i - D));
     __syncthreads();
   }
   float* cands = rows + M::ROWS_FLOATS + M::LAM_FLOATS;
@@ -391,7 +408,14 @@ ant_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const float*
     float2 a;
     if (ROLL) {  // the policy reads the observation the previous pass staged in shared memory (sobs is dense: [EPW][D])
       float* scr = cands + es * 128;
-      a = ra.H == 64 ? mlp_policy<16>(wsm, D, sobs + es * D, scr, k) : mlp_policy<8>(wsm, D, sobs + es * D, scr, k);
+      const float* x = sobs + es * D;
+      if (ROLL == 2) {  // normalized input in the scratch's upper half: layer 1 reads it, layer 2 overwrites it; sobs stays raw
+        HRL_CHECK(D <= 64 && es >= 0 && es < EPW);
+        for (int i = l; i < D; i += LPE) scr[64 + i] = norm_obs(sobs[es * D + i], nstat, D, i, ra.obs_clip);
+        __syncwarp();
+        x = scr + 64;
+      }
+      a = ra.H == 64 ? mlp_policy<16>(wsm, D, x, scr, k) : mlp_policy<8>(wsm, D, x, scr, k);
       if (ra.sigma_v || ra.sigma > 0.f) {  // exploration noise: Box-Muller on the counter RNG, keyed by (seed, env), addressed by the env's step count
         const float s1 = ra.sigma_v ? __ldg(ra.sigma_v + 2 * k) : ra.sigma, s2 = ra.sigma_v ? __ldg(ra.sigma_v + 2 * k + 1) : ra.sigma;
         float u[4];
@@ -1012,6 +1036,7 @@ __device__ __forceinline__ float2 mlp_policy16(const float* __restrict__ w, int 
 // ROLL = 1: the fused rollout of PointGather (see ant_env_kernel): step -1 composes the initial observation, steps
 // 0 .. T-1 are full steps whose actions the MLP computes from the observation the previous pass left in sobs; the env
 // state stays in registers in between.  Dynamic shared memory: [EPB][64] hidden activations, then the weights.
+// ROLL = 2: ROLL = 1 with a normalized policy input (hrl_rollout_mlp_norm); mean[D] and rstd[D] follow the weights.
 template <int ROLL = 0>
 __global__ void __launch_bounds__(16 * HRL_POINT_EPB)
 point_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const float* __restrict__ actions,
@@ -1029,10 +1054,13 @@ point_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const floa
   const uint32_t genv = (uint32_t)(cfg.env_index_offset + e);
   float* hid = smem + eb * 64;
   const float* wsm = smem + HRL_POINT_EPB * 64;
+  const float* nstat = wsm + (ROLL == 2 ? D * ra.H + ra.H + ra.H * ra.H + ra.H + ra.H * 2 + 2 : 0);  // ROLL = 2: mean[D], rstd[D]
   if (ROLL) {
     HRL_CHECK(D <= HRL_POINT_OBS && (ra.H == 32 || ra.H == 64));
     const int nw = D * ra.H + ra.H + ra.H * ra.H + ra.H + ra.H * 2 + 2;
     for (int i = threadIdx.x; i < nw; i += 16 * HRL_POINT_EPB) const_cast<float*>(wsm)[i] = __ldg(ra.w + i);
+    if (ROLL == 2)
+      for (int i = threadIdx.x; i < 2 * D; i += 16 * HRL_POINT_EPB) const_cast<float*>(nstat)[i] = __ldg(i < D ? ra.obs_mean + i : ra.obs_rstd + (i - D));
     __syncthreads();
   }
   const float4 b0 = st.base[e * 4 + 0], b2 = st.base[e * 4 + 2];
@@ -1054,7 +1082,15 @@ point_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const floa
   if (mode <= 1) {
     float ax, ay;
     if (ROLL) {
-      const float2 a = ra.H == 64 ? mlp_policy16<4>(wsm, D, sobs[eb], hid, j) : mlp_policy16<2>(wsm, D, sobs[eb], hid, j);
+      const float* x = sobs[eb];
+      if (ROLL == 2) {  // normalized input in this env's sensor-bin tile (64 floats), which the observation pass re-initialises
+        static_assert(sizeof(sb[0]) >= HRL_POINT_OBS * sizeof(float), "the bin tile must hold a normalized observation");
+        float* xn = reinterpret_cast<float*>(sb[eb]);
+        for (int i = j; i < D; i += 16) xn[i] = norm_obs(sobs[eb][i], nstat, D, i, ra.obs_clip);
+        __syncwarp();
+        x = xn;
+      }
+      const float2 a = ra.H == 64 ? mlp_policy16<4>(wsm, D, x, hid, j) : mlp_policy16<2>(wsm, D, x, hid, j);
       ax = a.x; ay = a.y;
       if (ra.sigma_v || ra.sigma > 0.f) {  // exploration noise: one Box-Muller pair for the two components (as lane 0 of an ant)
         const float s1 = ra.sigma_v ? __ldg(ra.sigma_v) : ra.sigma, s2 = ra.sigma_v ? __ldg(ra.sigma_v + 1) : ra.sigma;
@@ -1525,6 +1561,12 @@ int hrl_create(const hrl_config* cfg, int32_t device, hrl_handle** out) {
   CKH(cudaFuncSetAttribute(ant_env_kernel<1, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, roll_smem));
   CKH(cudaFuncSetAttribute(ant_env_kernel<0, 1, 1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   CKH(cudaFuncSetAttribute(ant_env_kernel<1, 1, 1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  // normalized policy input: the observation mean and rstd (2 x obs_dim <= 120 floats) behind the weights
+  const int norm_smem = roll_smem + 2 * HRL_OBS_STAGE * (int)sizeof(float);
+  CKH(cudaFuncSetAttribute(ant_env_kernel<0, 1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, norm_smem));
+  CKH(cudaFuncSetAttribute(ant_env_kernel<1, 1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, norm_smem));
+  CKH(cudaFuncSetAttribute(ant_env_kernel<0, 1, 2>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  CKH(cudaFuncSetAttribute(ant_env_kernel<1, 1, 2>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   h->sub = default_sub();
   {
     // CTAs (= warps of 8 envs) per wave: 6 per SM with the 14-wide rows (37.5 KB), 7 with the compact ones (30.1 KB, ~7 %
@@ -1710,38 +1752,59 @@ int hrl_flagrun_next_target(hrl_handle* h, const uint8_t* d_mask, void* stream) 
   return HRL_OK;
 }
 
-/* Fused rollout: T env steps in ONE launch with an in-kernel MLP policy (see mlp_policy / mlp_policy16). */
-int hrl_rollout_mlp_ex(hrl_handle* h, int32_t T, const float* d_weights, int32_t hidden, float sigma, const float* d_sigma,
-                       uint64_t noise_seed, float* d_obs, float* d_act, float* d_rew, uint8_t* d_done, float* d_info,
-                       float* d_terminal_obs, void* stream) {
+/* Fused rollout: T env steps in ONE launch with an in-kernel MLP policy (see mlp_policy / mlp_policy16); with the
+ * observation statistics, the ROLL = 2 instantiations feed the policy the normalized observation (norm_obs). */
+int hrl_rollout_mlp_norm(hrl_handle* h, int32_t T, const float* d_weights, int32_t hidden, float sigma, const float* d_sigma,
+                         uint64_t noise_seed, const float* d_obs_mean, const float* d_obs_rstd, float obs_clip, float* d_obs,
+                         float* d_act, float* d_rew, uint8_t* d_done, float* d_info, float* d_terminal_obs, void* stream) {
   if (!h || T < 1 || !d_weights || !d_obs || !d_act || !d_rew || !d_done) return set_err(HRL_E_INVALID, "bad argument to hrl_rollout_mlp");
   if (hidden != 32 && hidden != 64) return set_err(HRL_E_INVALID, "hrl_rollout_mlp: hidden width must be 32 or 64");
   if (!(sigma >= 0.f)) return set_err(HRL_E_INVALID, "hrl_rollout_mlp: sigma must be >= 0");
+  if (!d_obs_mean != !d_obs_rstd)
+    return set_err(HRL_E_INVALID, "hrl_rollout_mlp_norm: d_obs_mean and d_obs_rstd must both be given or both be NULL");
+  const bool norm = d_obs_mean != nullptr;
+  if (norm && !(obs_clip > 0.f && isfinite(obs_clip)))
+    return set_err(HRL_E_INVALID, "hrl_rollout_mlp_norm: obs_clip must be finite and > 0");
   ON_DEVICE(h->device);
   DevState st = h->st;
   st.fin_flag = nullptr;
   RollArgs ra;
   ra.T = T; ra.H = hidden; ra.w = d_weights; ra.sigma = sigma; ra.sigma_v = d_sigma; ra.seed = noise_seed; ra.act_out = d_act;
-  const int nw = h->D * hidden + hidden + hidden * hidden + hidden + hidden * h->A + h->A;
+  ra.obs_mean = d_obs_mean; ra.obs_rstd = d_obs_rstd; ra.obs_clip = obs_clip;
+  const int nw = h->D * hidden + hidden + hidden * hidden + hidden + hidden * h->A + h->A + (norm ? 2 * h->D : 0);
   cudaStream_t s = (cudaStream_t)stream;
   if (h->cfg.env_kind == HRL_POINT_GATHER) {
     const int G = (h->N + HRL_POINT_EPB - 1) / HRL_POINT_EPB;
     const size_t smem = ((size_t)HRL_POINT_EPB * 64 + nw) * sizeof(float);
-    point_env_kernel<1><<<G, 16 * HRL_POINT_EPB, smem, s>>>(h->cfg, st, nullptr, nullptr, d_obs, d_rew, d_done, d_info, d_terminal_obs, 0, 0,
-                                                            h->D, ra);
+    if (norm)
+      point_env_kernel<2><<<G, 16 * HRL_POINT_EPB, smem, s>>>(h->cfg, st, nullptr, nullptr, d_obs, d_rew, d_done, d_info, d_terminal_obs, 0, 0,
+                                                              h->D, ra);
+    else
+      point_env_kernel<1><<<G, 16 * HRL_POINT_EPB, smem, s>>>(h->cfg, st, nullptr, nullptr, d_obs, d_rew, d_done, d_info, d_terminal_obs, 0, 0,
+                                                              h->D, ra);
   } else {
     const int Tn = 32 * HRL_ROLL_WARPS, EPC = Map<1>::EPW * HRL_ROLL_WARPS, G = (h->N + EPC - 1) / EPC;
     const size_t smem = ((size_t)HRL_ROLL_WARPS * Map<1>::SMEM_FLOATS + nw) * sizeof(float);
-    if (h->cfg.env_kind == HRL_ANT_GATHER)
-      ant_env_kernel<0, 1, 1><<<G, Tn, smem, s>>>(h->cfg, st, h->d_bounds, h->n_lines, nullptr, nullptr, d_obs, d_rew, d_done, d_info,
-                                                  d_terminal_obs, 0, 0, h->D, ra);
-    else
-      ant_env_kernel<1, 1, 1><<<G, Tn, smem, s>>>(h->cfg, st, h->d_bounds, h->n_lines, nullptr, nullptr, d_obs, d_rew, d_done, d_info,
-                                                  d_terminal_obs, 0, 0, h->D, ra);
+#define ROLL_LAUNCH(FAM, R)                                                                                                 \
+  ant_env_kernel<FAM, 1, R><<<G, Tn, smem, s>>>(h->cfg, st, h->d_bounds, h->n_lines, nullptr, nullptr, d_obs, d_rew, d_done, d_info, \
+                                                d_terminal_obs, 0, 0, h->D, ra)
+    if (h->cfg.env_kind == HRL_ANT_GATHER) {
+      if (norm) ROLL_LAUNCH(0, 2); else ROLL_LAUNCH(0, 1);
+    } else {
+      if (norm) ROLL_LAUNCH(1, 2); else ROLL_LAUNCH(1, 1);
+    }
+#undef ROLL_LAUNCH
   }
   g_launches++;
   CK(cudaGetLastError());
   return HRL_OK;
+}
+
+int hrl_rollout_mlp_ex(hrl_handle* h, int32_t T, const float* d_weights, int32_t hidden, float sigma, const float* d_sigma,
+                       uint64_t noise_seed, float* d_obs, float* d_act, float* d_rew, uint8_t* d_done, float* d_info,
+                       float* d_terminal_obs, void* stream) {
+  return hrl_rollout_mlp_norm(h, T, d_weights, hidden, sigma, d_sigma, noise_seed, nullptr, nullptr, 0.f, d_obs, d_act, d_rew, d_done,
+                              d_info, d_terminal_obs, stream);
 }
 
 int hrl_rollout_mlp(hrl_handle* h, int32_t T, const float* d_weights, int32_t hidden, float sigma, uint64_t noise_seed, float* d_obs,
@@ -1815,6 +1878,82 @@ int hrl_gae(int32_t T, int32_t N, float gamma, float lam, const float* d_rew, co
   const int W = gae_warps(T, N, sms), L = (T + W - 1) / W;
   gae_kernel<<<(N + 31) / 32, 32 * W, 0, (cudaStream_t)stream>>>(T, N, L, gamma, gamma * lam, d_rew, d_done, d_info, d_values,
                                                                  d_terminal_values, d_adv, d_ret);
+  g_launches++;
+  CK(cudaGetLastError());
+  return HRL_OK;
+}
+
+// CTAs of the one-cluster normalization kernels (hrl_normalize.cuh) on the current device: 16 (a non-portable cluster
+// size) where the device can co-schedule them, else the portable 8.  Cached per device.
+static int norm_cluster_size(int dev) {
+  static std::atomic<int> cache[64];
+  if (dev >= 0 && dev < 64 && cache[dev].load()) return cache[dev].load();
+  int best = 8;
+  const void* kernels[2] = {(const void*)obs_moments_kernel, (const void*)return_moments_kernel};
+  bool ok16 = true;
+  for (const void* k : kernels) {
+    ok16 = ok16 && cudaFuncSetAttribute(k, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(16); cfg.blockDim = dim3(HRL_NORM_THREADS);
+    cudaLaunchAttribute a;
+    a.id = cudaLaunchAttributeClusterDimension;
+    a.val.clusterDim.x = 16; a.val.clusterDim.y = 1; a.val.clusterDim.z = 1;
+    cfg.attrs = &a; cfg.numAttrs = 1;
+    int n = 0;
+    ok16 = ok16 && cudaOccupancyMaxActiveClusters(&n, k, &cfg) == cudaSuccess && n >= 1;
+  }
+  cudaGetLastError();  // a refused query is an answer, not an error of the next launch
+  if (ok16) best = 16;
+  if (dev >= 0 && dev < 64) cache[dev].store(best);
+  return best;
+}
+
+extern "C++" {  // a template cannot have C linkage
+template <typename... Exp, typename... Act>
+static cudaError_t launch_cluster(void (*kernel)(Exp...), int C, cudaStream_t s, Act&&... args) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(C); cfg.blockDim = dim3(HRL_NORM_THREADS); cfg.dynamicSmemBytes = 0; cfg.stream = s;
+  cudaLaunchAttribute a;
+  a.id = cudaLaunchAttributeClusterDimension;
+  a.val.clusterDim.x = C; a.val.clusterDim.y = 1; a.val.clusterDim.z = 1;
+  cfg.attrs = &a; cfg.numAttrs = 1;
+  return cudaLaunchKernelEx(&cfg, kernel, std::forward<Act>(args)...);
+}
+}
+
+/* Running observation statistics (obs_moments_kernel, hrl_normalize.cuh); runs on the current device. */
+int hrl_obs_moments(int32_t M, int32_t D, const float* d_x, double* d_moments, float eps, float* d_mean_f, float* d_rstd_f,
+                    void* stream) {
+  if (M < 1 || D < 1 || D > HRL_NORM_MAX_D || !d_x || !d_moments || !d_mean_f || !d_rstd_f)
+    return set_err(HRL_E_INVALID, "bad argument to hrl_obs_moments");
+  if (!(eps > 0.f)) return set_err(HRL_E_INVALID, "hrl_obs_moments: eps must be > 0");
+  int dev = 0;
+  CK(cudaGetDevice(&dev));
+  const int C = norm_cluster_size(dev);
+  CK(launch_cluster(obs_moments_kernel, C, (cudaStream_t)stream, (int)M, (int)D, d_x, d_moments, eps, d_mean_f, d_rstd_f));
+  g_launches++;
+  return HRL_OK;
+}
+
+/* Return-based reward scaling (return_scan_kernel, return_moments_kernel, reward_apply_kernel); current device. */
+int hrl_reward_scale(int32_t T, int32_t N, float gamma, float clip, float eps, const float* d_rew, const uint8_t* d_done,
+                     double* d_returns, double* d_ret_moments, double* d_work, float* d_out, void* stream) {
+  if (T < 1 || N < 1 || !d_rew || !d_done || !d_returns || !d_ret_moments || !d_work || !d_out)
+    return set_err(HRL_E_INVALID, "bad argument to hrl_reward_scale");
+  if (!(gamma >= 0.f && gamma <= 1.f)) return set_err(HRL_E_INVALID, "hrl_reward_scale: gamma must lie in [0, 1]");
+  if (!(clip > 0.f) || !(eps > 0.f)) return set_err(HRL_E_INVALID, "hrl_reward_scale: clip and eps must be > 0");
+  int dev = 0, sms = 0;
+  CK(cudaGetDevice(&dev));
+  CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  const int C = norm_cluster_size(dev);
+  cudaStream_t s = (cudaStream_t)stream;
+  return_scan_kernel<<<(N + 255) / 256, 256, 0, s>>>(T, N, (double)gamma, d_rew, d_done, d_returns, d_out);
+  g_launches++;
+  CK(cudaGetLastError());
+  CK(launch_cluster(return_moments_kernel, C, s, (int)T, (int)N, eps, (const float*)d_out, d_ret_moments, d_work));
+  g_launches++;
+  const int gx = (N + 255) / 256, gy = (int)std::min<long long>(T, std::max<long long>(1, 8LL * sms / gx));
+  reward_apply_kernel<<<dim3(gx, gy), 256, 0, s>>>(T, N, clip, d_rew, d_work, d_out);
   g_launches++;
   CK(cudaGetLastError());
   return HRL_OK;

@@ -124,7 +124,7 @@ class RolloutBuffer:
             raise ValueError("this RolloutBuffer holds no info (create it with info=True)")
         return LazyInfo(self.info[t], self.kind, None if self.terminal_obs is None else self.terminal_obs[t])
 
-    def gae(self, values, gamma=0.99, lam=0.95, terminal_values=None, out=None):
+    def gae(self, values, gamma=0.99, lam=0.95, terminal_values=None, out=None, rew=None):
         """GAE(lambda) advantages and returns of the T steps in this buffer, in ONE kernel launch (include/hrl_b200.h
         `hrl_gae`).  ``values``: float32 [T + 1, N], V(obs[0..T]).  ``terminal_values``: float32 [T, N], typically
         ``critic(buf.terminal_obs)`` over the whole tensor (stale rows included: a row is read only where it is selected);
@@ -132,7 +132,8 @@ class RolloutBuffer:
         ``terminal_values[t]`` and one ended by the env from 0; without it, every done is a termination.  ``obs[t + 1]`` of
         an env that finished in step t is the reset observation, so its value never bootstraps step t.
         ``out=(adv, ret)``: float32 [T, N] tensors written in place (no allocation, so the call can be captured in a CUDA
-        graph).  No host synchronisation.  Returns ``(adv, ret)``."""
+        graph).  ``rew``: float32 [T, N] rewards used instead of ``self.rew`` (e.g. ``RunningNormalizer.scale_rewards``).
+        No host synchronisation.  Returns ``(adv, ret)``."""
         T, N = self.rew.shape
         dev = self.rew.device
 
@@ -142,6 +143,10 @@ class RolloutBuffer:
                 raise ValueError("%s must be a contiguous float32 tensor [%s] on %s" % (name, ", ".join(map(str, shape)), dev))
 
         check("values", values, (T + 1, N))
+        if rew is not None:
+            check("rew", rew, (T, N))
+        else:
+            rew = self.rew
         if terminal_values is not None:
             if self.info is None:
                 raise ValueError("terminal_values need the truncation flags: create the RolloutBuffer with info=True")
@@ -158,7 +163,7 @@ class RolloutBuffer:
             check("out[1] (ret)", ret, (T, N))
         info = self.info if terminal_values is not None else None
         with torch.cuda.device(dev):
-            _cabi.check(_cabi.lib().hrl_gae(T, N, float(gamma), float(lam), _ptr(self.rew), _ptr(self.done), _ptr(info), _ptr(values),
+            _cabi.check(_cabi.lib().hrl_gae(T, N, float(gamma), float(lam), _ptr(rew), _ptr(self.done), _ptr(info), _ptr(values),
                                             _ptr(terminal_values), _ptr(adv), _ptr(ret),
                                             C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
         return adv, ret
@@ -322,12 +327,15 @@ class VecEnv:
             parts += [W.detach().to(torch.float32).t().contiguous().reshape(-1), b.detach().to(torch.float32).reshape(-1)]
         return torch.cat(parts).contiguous()
 
-    def rollout_mlp(self, layers, horizon, buf=None, sigma=0.0, noise_seed=0, want_info=False, want_terminal_obs=False):
+    def rollout_mlp(self, layers, horizon, buf=None, sigma=0.0, noise_seed=0, want_info=False, want_terminal_obs=False,
+                    obs_norm=None):
         """Fused rollout (include/hrl_b200.h `hrl_rollout_mlp_ex`): `horizon` steps in ONE kernel launch, actions from the
         3-layer tanh MLP `layers` = ((W1[H, D], b1), (W2[H, H], b2), (W3[A, H], b3)) evaluated inside the kernel (H = 32 or
         64), plus N(0, sigma^2) exploration noise.  `sigma` is a float or a length-A tensor (one scale per action
         component, e.g. exp(log_std) of a Gaussian policy).  Fills and returns a RolloutBuffer: obs[0..T], act, rew,
-        done, and with `want_info` / `want_terminal_obs` also info / terminal_obs (allocated when `buf` is None)."""
+        done, and with `want_info` / `want_terminal_obs` also info / terminal_obs (allocated when `buf` is None).
+        `obs_norm`: a `RunningNormalizer` of this env's obs_dim; the policy then reads `obs_norm.normalize(obs)`, with the
+        statistics frozen for the launch (`hrl_rollout_mlp_norm`).  The buffer still receives the raw observations."""
         (W1, b1), (W2, b2), (W3, b3) = layers
         H = W1.shape[0]
         if H not in (32, 64) or tuple(W1.shape) != (H, self.D) or tuple(W2.shape) != (H, H) or tuple(W3.shape) != (self.A, H):
@@ -341,6 +349,8 @@ class VecEnv:
             if not bool((torch.isfinite(sig_v) & (sig_v >= 0)).all()):
                 raise ValueError("sigma entries must be finite and >= 0")
             sigma = 0.0
+        if obs_norm is not None and (getattr(obs_norm, "D", None) != self.D or getattr(obs_norm, "device", None) != self.device):
+            raise ValueError("obs_norm must be a RunningNormalizer of obs_dim %d on %s" % (self.D, self.device))
         buf = buf or RolloutBuffer(self, horizon, info=want_info, terminal_obs=want_terminal_obs)
         if buf.T < horizon:
             raise ValueError("rollout buffer holds %d steps, need %d" % (buf.T, horizon))
@@ -350,9 +360,15 @@ class VecEnv:
         term = buf.terminal_obs if want_terminal_obs else None
         if _NVTX:
             torch.cuda.nvtx.range_push("hrl.rollout_mlp")
-        _cabi.check(self.L.hrl_rollout_mlp_ex(self.h, int(horizon), _ptr(w), int(H), float(sigma), _ptr(sig_v), int(noise_seed),
-                                              _ptr(buf.obs), _ptr(buf.act), _ptr(buf.rew), _ptr(buf.done), _ptr(info), _ptr(term),
-                                              self._stream()))
+        if obs_norm is None:
+            _cabi.check(self.L.hrl_rollout_mlp_ex(self.h, int(horizon), _ptr(w), int(H), float(sigma), _ptr(sig_v), int(noise_seed),
+                                                  _ptr(buf.obs), _ptr(buf.act), _ptr(buf.rew), _ptr(buf.done), _ptr(info), _ptr(term),
+                                                  self._stream()))
+        else:
+            _cabi.check(self.L.hrl_rollout_mlp_norm(self.h, int(horizon), _ptr(w), int(H), float(sigma), _ptr(sig_v), int(noise_seed),
+                                                    _ptr(obs_norm.mean), _ptr(obs_norm.rstd), obs_norm.clip_obs, _ptr(buf.obs),
+                                                    _ptr(buf.act), _ptr(buf.rew), _ptr(buf.done), _ptr(info), _ptr(term),
+                                                    self._stream()))
         if _NVTX:
             torch.cuda.nvtx.range_pop()
         self._keep = (w, sig_v)   # the launch is asynchronous: keep the packed weights and noise scales alive

@@ -226,6 +226,21 @@ int hrl_rollout_mlp_ex(hrl_handle* h, int32_t T, const float* d_weights, int32_t
                        uint64_t noise_seed, float* d_obs, float* d_act, float* d_rew, uint8_t* d_done, float* d_info,
                        float* d_terminal_obs, void* stream);
 
+/* hrl_rollout_mlp_ex with a normalized policy input (hrl_rollout_mlp_ex is this call with NULL, NULL, 0).
+ *   d_obs_mean, d_obs_rstd f32[obs_dim]: both NULL (the raw observation, as hrl_rollout_mlp_ex) or both non-NULL.  The
+ *   policy then reads, for obs component i,
+ *       x_i = fminf(fmaxf((o_i - mean_i) * rstd_i, -obs_clip), obs_clip)       (float32; subtract, multiply, clamp)
+ *   so torch.clamp((obs - mean) * rstd, -obs_clip, obs_clip) gives the same bits for finite observations.  obs_clip must be
+ *   finite and > 0 when the statistics are given.  The statistics are read once per launch: they are frozen for the T steps.
+ *   d_obs and d_terminal_obs still receive the RAW observations.
+ * The one difference from SB3 VecNormalize: SB3 updates the observation statistics every step, so step t + 1's input is
+ * normalized with statistics that already include it.  Here the statistics are frozen for a rollout and updated from its
+ * observations afterwards (hrl_obs_moments), as GPU-batched PPO implementations do. */
+int hrl_rollout_mlp_norm(hrl_handle* h, int32_t T, const float* d_weights, int32_t hidden, float sigma, const float* d_sigma,
+                         uint64_t noise_seed, const float* d_obs_mean, const float* d_obs_rstd, float obs_clip,
+                         float* d_obs, float* d_act, float* d_rew, uint8_t* d_done, float* d_info, float* d_terminal_obs,
+                         void* stream);
+
 /* Replaces saveState/restoreState (used as the reset mechanism by pybullet_envs) and gives
  * the "identical saved states" hook the one-step parity tests need.
  *   d_fstate f32[N, HRL_STATE_F], d_istate i32[N, HRL_STATE_I]. */
@@ -264,6 +279,32 @@ int hrl_sense_walls(int32_t M, int32_t n_bins, float span, float range, int32_t 
  * anything, NaN included.  d_adv / d_ret must not overlap the inputs. */
 int hrl_gae(int32_t T, int32_t N, float gamma, float lam, const float* d_rew, const uint8_t* d_done, const float* d_info,
             const float* d_values, const float* d_terminal_values, float* d_adv, float* d_ret, void* stream);
+/* Running observation statistics (SB3 RunningMeanStd; DESIGN.md section 4, kernel 8).  Stateless, current device.
+ * Merges the batch d_x f32[M, D] into d_moments f64[1 + 2D] = {count, mean[D], var[D]} with SB3's update_from_moments:
+ *   delta = bmean - mean;  tot = count + M;  mean += delta * M / tot;
+ *   var = (var * count + bvar * M + delta^2 * count * M / tot) / tot;  count = tot        (bvar: population variance)
+ * then writes d_mean_f[i] = (float)mean[i] and d_rstd_f[i] = (float)(1 / sqrt(var[i] + eps)), the two arrays
+ * hrl_rollout_mlp_norm reads.  The initial state is the caller's (SB3: count = 1e-4, mean = 0, var = 1).
+ * Accumulates in float64 (deviations from a sample inside a thread, Chan merges above it, in a fixed order); ONE launch of
+ * one thread-block cluster, no atomics, no scratch memory: the same inputs give the same bytes on every call, and calls on
+ * different streams may overlap.  No host synchronisation, no allocation: capturable in a CUDA graph.
+ * 1 <= M, 1 <= D <= 64, eps > 0, no NULL pointer. */
+int hrl_obs_moments(int32_t M, int32_t D, const float* d_x, double* d_moments, float eps, float* d_mean_f, float* d_rstd_f,
+                    void* stream);
+/* Return-based reward scaling with SB3 VecNormalize's sequential semantics (step_wait, _update_reward, normalize_reward).
+ * Stateless, current device.  For t = 0 .. T-1:
+ *   R[e]      = gamma * R[e] + rew[t, e]                                (d_returns f64[N], carried across calls)
+ *   moments   = merge(moments, mean_e R, population-var_e R, count N)    (d_ret_moments f64[3] = {count, mean, var})
+ *   s_t       = (float)(1 / sqrt(var + eps))
+ *   out[t, e] = fminf(fmaxf(rew[t, e] * s_t, -clip), clip)              (float32)
+ *   R[e]      = 0 where done[t, e]                                       (truncations included, as in SB3)
+ * R is kept in float64; the per-step mean and variance are taken over R rounded to float32 (a relative difference of at
+ * most 2^-24 per value).  d_rew f32[T, N], d_done u8[T, N], d_work f64 scratch of >= 2 T entries (contents on entry do not
+ * matter), d_out f32[T, N], which must not overlap the inputs.  1 <= T, N; 0 <= gamma <= 1; clip, eps > 0.
+ * THREE launches (a scan over T per env, one cluster for the statistics and the chain over t, the scaling), no atomics:
+ * the same bytes on every call.  No host synchronisation, capturable in a CUDA graph. */
+int hrl_reward_scale(int32_t T, int32_t N, float gamma, float clip, float eps, const float* d_rew, const uint8_t* d_done,
+                     double* d_returns, double* d_ret_moments, double* d_work, float* d_out, void* stream);
 /* `n_sub` physics sub-steps on the handle's current state (no task logic, no reset):
  * replaces scene.global_step() -> p.stepSimulation() (ant_gather_env.py:78). */
 int hrl_substeps(hrl_handle* h, const float* d_actions, int32_t n_sub, void* stream);
