@@ -28,7 +28,7 @@
 #ifndef HRL_WARPS_PER_CTA
 #define HRL_WARPS_PER_CTA 1
 #endif
-#define HRL_OBS_STAGE 64  // floats per env in the staging tile (max obs dim 60)
+#define HRL_OBS_STAGE 64  // floats per env in the staging tile = the widest observation hrl_create accepts
 
 // ------------------------------------------------------------------------------------------
 // device state (internal SoA layout; the public layout of hrl_get_state is converted by kernels)
@@ -298,7 +298,7 @@ __device__ __forceinline__ float norm_obs(float o, const float* __restrict__ sta
   return fminf(fmaxf(__fmul_rn(__fsub_rn(o, stat[i]), stat[D + i]), -clip), clip);
 }
 #define HRL_ROLL_WARPS 2                       // warps per CTA of the fused-rollout instantiations (they share the weights)
-#define HRL_MLP_MAX_FLOATS (60 * 64 + 64 + 64 * 64 + 64 + 64 * 8 + 8)   // obs_dim <= 60, H <= 64
+#define HRL_MLP_MAX_FLOATS (HRL_OBS_STAGE * 64 + 64 + 64 * 64 + 64 + 64 * 8 + 8)   // obs_dim <= HRL_OBS_STAGE, H <= 64
 
 #ifdef HRL_DEBUG_CONTACTS
 __device__ float* g_dbg_contacts = nullptr;  // [N][4 legs][40]: candidate lists of the first sub-step of the last launch
@@ -1555,13 +1555,13 @@ int hrl_create(const hrl_config* cfg, int32_t device, hrl_handle** out) {
   CKH(cudaFuncSetAttribute(ant_env_kernel<FAM, SUB>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared))
   OPT_IN(0, 0); OPT_IN(1, 0); OPT_IN(0, 1); OPT_IN(1, 1); OPT_IN(0, 2); OPT_IN(1, 2); OPT_IN(0, 4); OPT_IN(1, 4);
 #undef OPT_IN
-  // the fused-rollout instantiations: 2 warps per CTA + the policy weights (<= 34 KB) in shared memory, 2 CTAs per SM
+  // the fused-rollout instantiations: 2 warps per CTA + the policy weights (<= 35 KB) in shared memory, 2 CTAs per SM
   const int roll_smem = (HRL_ROLL_WARPS * Map<1>::SMEM_FLOATS + HRL_MLP_MAX_FLOATS) * (int)sizeof(float);
   CKH(cudaFuncSetAttribute(ant_env_kernel<0, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, roll_smem));
   CKH(cudaFuncSetAttribute(ant_env_kernel<1, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, roll_smem));
   CKH(cudaFuncSetAttribute(ant_env_kernel<0, 1, 1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   CKH(cudaFuncSetAttribute(ant_env_kernel<1, 1, 1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  // normalized policy input: the observation mean and rstd (2 x obs_dim <= 120 floats) behind the weights
+  // normalized policy input: the observation mean and rstd (2 x obs_dim <= 2 x HRL_OBS_STAGE floats) behind the weights
   const int norm_smem = roll_smem + 2 * HRL_OBS_STAGE * (int)sizeof(float);
   CKH(cudaFuncSetAttribute(ant_env_kernel<0, 1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, norm_smem));
   CKH(cudaFuncSetAttribute(ant_env_kernel<1, 1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, norm_smem));

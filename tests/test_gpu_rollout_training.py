@@ -47,7 +47,12 @@ def _twins(env_id, N, pre_steps=3, **kw):
 # observation is then the one composed with the new goal, before the reset (the reference's ordering)
 REPLAY_CASES = [("AntGatherBulletEnv-v0", 64, {}), ("AntMazeBulletEnv-v0", 32, {}), ("AntFlagrunBulletEnv-v0", 64, {}),
                 ("AntFlagrunBulletEnv-v0", 32, dict(timeout=5)), ("AntMjBulletEnv-v0", 64, {}), ("PointGatherBulletEnv-v0", 64, {}),
-                ("PointGatherBulletEnv-v0", 32, dict(use_sensor=False))]
+                ("PointGatherBulletEnv-v0", 32, dict(use_sensor=False)),
+                # cube colliders and contact pickup inside the rollout; the widest observations (AntMazeMj n_bins = 11: D = 63)
+                ("AntGatherBulletEnv-v0", 64, dict(robot_coll_dist=0)), ("AntGatherBulletEnv-v0", 32, dict(n_bins=16)),
+                ("AntMazeBulletEnv-v0", 64, dict(sense_target=True)), ("AntMazeBulletEnv-v0", 32, dict(max_steps=20, done_at_target=False)),
+                ("AntMazeMjEnv-v0", 32, {}), ("AntMazeMjEnv-v0", 64, dict(n_bins=11)), ("AntFlagrunBulletEnv-v0", 64, dict(use_sensor=True)),
+                ("AntFlagrunBulletEnv-v0", 32, dict(max_targets=0, max_target_dist=4)), ("AntFlagrunBulletEnv-v0", 64, dict(enclosed=False))]
 
 
 @pytest.mark.parametrize("env_id,H,kw", REPLAY_CASES)
@@ -192,4 +197,4 @@ def test_bounds_checked_build_runs_rollouts_clean():
                        text=True, timeout=600)
     assert r.returncode == 0, (r.stdout[-2000:], r.stderr[-3000:])
     assert "bounds rollout run complete" in r.stdout
-    assert r.stdout.count("ok ") >= 16
+    assert r.stdout.count("ok ") >= 20

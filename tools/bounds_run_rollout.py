@@ -11,6 +11,7 @@ assert b"HRL_BOUNDS" in _cabi.lib().hrl_version(), "not the bounds-checked build
 N, T = 203, 16   # ragged last CTA of both kernels
 CASES = [("AntGatherBulletEnv-v0", {}), ("AntGatherBulletEnv-v0", dict(use_sensor=False)), ("AntMazeBulletEnv-v0", dict(sense_target=True)),
          ("AntFlagrunBulletEnv-v0", dict(timeout=4)), ("AntMjBulletEnv-v0", {}), ("AntMazeMjEnv-v0", {}),
+         ("AntMazeMjEnv-v0", dict(n_bins=11)), ("AntGatherBulletEnv-v0", dict(robot_coll_dist=0)),
          ("PointGatherBulletEnv-v0", {}), ("PointGatherBulletEnv-v0", dict(use_sensor=False, n_bins=16))]
 g = torch.Generator().manual_seed(5)
 for env_id, kw in CASES:
