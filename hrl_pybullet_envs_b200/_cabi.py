@@ -26,7 +26,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
 # every symbol include/hrl_b200.h declares (checked by tests/test_cabi_symbols.py)
 SYMBOLS = ["hrl_default_config", "hrl_obs_dim", "hrl_act_dim", "hrl_create", "hrl_destroy", "hrl_reset", "hrl_step",
            "hrl_step_host", "hrl_set_host_mode", "hrl_host_layout", "hrl_get_state", "hrl_set_state", "hrl_observe", "hrl_gather_sensor", "hrl_sense_walls", "hrl_gae",
-           "hrl_obs_moments", "hrl_reward_scale", "hrl_substeps", "hrl_rollout_mlp", "hrl_rollout_mlp_ex", "hrl_rollout_mlp_norm", "hrl_flagrun_next_target", "hrl_get_stats", "hrl_stream_gate", "hrl_set_lanes_per_env", "hrl_get_lanes_per_env", "hrl_set_compact_rows",
+           "hrl_obs_moments", "hrl_reward_scale", "hrl_substeps", "hrl_rollout_mlp", "hrl_rollout_mlp_ex", "hrl_rollout_mlp_norm", "hrl_evaluate_mlp", "hrl_flagrun_next_target", "hrl_get_stats", "hrl_stream_gate", "hrl_set_lanes_per_env", "hrl_get_lanes_per_env", "hrl_set_compact_rows",
            "hrl_get_compact_rows", "hrl_launch_count", "hrl_last_error", "hrl_version"]
 
 
@@ -83,6 +83,7 @@ def lib():
     L.hrl_rollout_mlp.argtypes = [vp, i32, vp, i32, f32, C.c_uint64, vp, vp, vp, vp, vp]
     L.hrl_rollout_mlp_ex.argtypes = [vp, i32, vp, i32, f32, vp, C.c_uint64, vp, vp, vp, vp, vp, vp, vp]
     L.hrl_rollout_mlp_norm.argtypes = [vp, i32, vp, i32, f32, vp, C.c_uint64, vp, vp, f32, vp, vp, vp, vp, vp, vp, vp]
+    L.hrl_evaluate_mlp.argtypes = [vp, i32, i32, vp, i32, f32, vp, C.c_uint64, vp, vp, f32, vp, vp, vp, vp]
     L.hrl_obs_moments.argtypes = [i32, i32, vp, vp, f32, vp, vp, vp]
     L.hrl_reward_scale.argtypes = [i32, i32, f32, f32, f32] + [vp] * 7
     L.hrl_flagrun_next_target.argtypes = [vp, vp, vp]

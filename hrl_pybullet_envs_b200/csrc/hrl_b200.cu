@@ -81,6 +81,10 @@ static int set_err(int code, const char* msg) {
   snprintf(g_err, sizeof g_err, "%s", msg);
   return code;
 }
+static int set_err(int code, const char* fn, const char* msg) {  // "fn: msg"
+  snprintf(g_err, sizeof g_err, "%s: %s", fn, msg);
+  return code;
+}
 static int cuda_fail(cudaError_t e, const char* where) {
   snprintf(g_err, sizeof g_err, "%s: %s", where, cudaGetErrorString(e));
   return HRL_E_CUDA;
@@ -243,6 +247,12 @@ struct RollArgs {
   const float* obs_mean;  // [D]
   const float* obs_rstd;  // [D]
   float obs_clip;
+  // members (hrl_evaluate_mlp): env e runs the policy at w + (e / m_envs) * nw; a CTA holds envs of one member only
+  int m_envs;
+  // per-env results over the launch up to the first done (hrl_evaluate_mlp), or NULL: return, length, finished flag
+  float* ev_ret;
+  int32_t* ev_len;
+  uint8_t* ev_fin;
 };
 enum { STREAM_POLICY = 6 };
 
@@ -323,7 +333,8 @@ ant_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const float*
   const float* nstat = wsm + (ROLL == 2 ? D * ra.H + ra.H + ra.H * ra.H + ra.H + ra.H * 8 + 8 : 0);
   if (ROLL) {
     const int nw = D * ra.H + ra.H + ra.H * ra.H + ra.H + ra.H * 8 + 8;
-    for (int i = threadIdx.x; i < nw; i += 32 * WPC) const_cast<float*>(wsm)[i] = __ldg(ra.w + i);
+    const float* wg = ra.w + (size_t)((int)blockIdx.x * WPC * EPW / ra.m_envs) * nw;   // this CTA's member
+    for (int i = threadIdx.x; i < nw; i += 32 * WPC) const_cast<float*>(wsm)[i] = __ldg(wg + i);
     if (ROLL == 2)
       for (int i = threadIdx.x; i < 2 * D; i += 32 * WPC) const_cast<float*>(nstat)[i] = __ldg(i < D ? ra.obs_mean + i : ra.obs_rstd + (i - D));
     __syncthreads();
@@ -366,6 +377,10 @@ ant_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const float*
     T.feet[0] = m1.x; T.feet[1] = m1.y; T.feet[2] = m1.z; T.feet[3] = m1.w;
     T.t = i0.x; T.episode = i0.y; T.steps_total = i0.z; T.goals_left = i0.w; T.since = i1.x; T.rewarded = i1.y; T.gen = i1.z;
   }
+  // ROLL: the launch's first episode - its return (rewards added in step order) and length ev_n while it runs, ~length
+  // once a done has ended it (one register for the length and the flag)
+  float ev_ret = 0.f;
+  int ev_n = 0;
   float it_x[IPL], it_y[IPL];  // this lane's items IPL * l .. IPL * l + IPL - 1 (food 0-7, poison 8-15)
   if (FAMILY == 0) {
     if (IPL == 4) {
@@ -385,9 +400,10 @@ ant_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const float*
 #pragma unroll 1
   for (int step = ROLL ? -1 : 0; step < (ROLL ? ra.T : 1); step++) {
   const int mode = ROLL ? (step < 0 ? 3 : 0) : mode_g;
-  float* __restrict__ obs_out = ROLL ? obs_out_g + (size_t)(step + 1) * N * D : obs_out_g;
-  float* __restrict__ rew_out = ROLL ? rew_out_g + (size_t)max(step, 0) * N : rew_out_g;
-  uint8_t* __restrict__ done_out = ROLL ? done_out_g + (size_t)max(step, 0) * N : done_out_g;
+  // ROLL: every per-step buffer may be NULL (hrl_evaluate_mlp passes none)
+  float* __restrict__ obs_out = ROLL && obs_out_g ? obs_out_g + (size_t)(step + 1) * N * D : obs_out_g;
+  float* __restrict__ rew_out = ROLL && rew_out_g ? rew_out_g + (size_t)max(step, 0) * N : rew_out_g;
+  uint8_t* __restrict__ done_out = ROLL && done_out_g ? done_out_g + (size_t)max(step, 0) * N : done_out_g;
   float* __restrict__ info_out = ROLL && info_out_g ? info_out_g + (size_t)max(step, 0) * N * 4 : info_out_g;
   float* __restrict__ term_out = ROLL && term_out_g ? term_out_g + (size_t)max(step, 0) * N * D : term_out_g;
   const float* __restrict__ bounds = bounds_g;
@@ -425,7 +441,7 @@ ant_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const float*
         sincosf(6.2831853f * u[1], &sn, &cs);
         a.x += s1 * r0 * cs; a.y += s2 * r0 * sn;
       }
-      if (active && sub == 0) reinterpret_cast<float2*>(ra.act_out)[((size_t)step * N + e) * 4 + k] = a;
+      if (active && sub == 0 && ra.act_out) reinterpret_cast<float2*>(ra.act_out)[((size_t)step * N + e) * 4 + k] = a;
     } else {
       a = reinterpret_cast<const float2*>(actions)[e * 4 + k];
     }
@@ -694,9 +710,10 @@ ant_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const float*
         if (cfg.max_episode_steps > 0 && T.t >= cfg.max_episode_steps) { trunc = done ? 0.f : 1.f; done = 1; }
         T.ret += food_rew + dead_rew;
         if (done) { T.ret_sum += T.ret; T.ret = 0.f; }
+        if (ROLL && ev_n >= 0) { ev_ret += food_rew + dead_rew; ev_n = done ? ~(ev_n + 1) : ev_n + 1; }
         if (active && l == 0) {
-          rew_out[e] = food_rew + dead_rew;
-          done_out[e] = (uint8_t)done;
+          if (!ROLL || rew_out) rew_out[e] = food_rew + dead_rew;
+          if (!ROLL || done_out) done_out[e] = (uint8_t)done;
           if (info_out) reinterpret_cast<float4*>(info_out)[e] = make_float4(food_rew, dead_rew, trunc, (float)T.t);
         }
       }
@@ -815,9 +832,10 @@ ant_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const float*
         if (cfg.max_episode_steps > 0 && T.t >= cfg.max_episode_steps) { trunc = done ? 0.f : 1.f; done = 1; }
         T.ret += rew;
         if (done) { T.ret_sum += T.ret; T.ret = 0.f; }
+        if (ROLL && ev_n >= 0) { ev_ret += rew; ev_n = done ? ~(ev_n + 1) : ev_n + 1; }
         if (active && l == 0) {
-          rew_out[e] = rew;
-          done_out[e] = (uint8_t)done;
+          if (!ROLL || rew_out) rew_out[e] = rew;
+          if (!ROLL || done_out) done_out[e] = (uint8_t)done;
           // info[2]: bit 0 = TimeLimit.truncated, bit 1 = the walk target changed in this step (info['target'] is set)
           if (info_out) reinterpret_cast<float4*>(info_out)[e] = make_float4(inner, info1, trunc + 2.f * (float)next, (float)T.t);
         }
@@ -867,8 +885,8 @@ ant_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const float*
         if (env0 + w8 < N && ((wmask >> (LPE * w8)) & 1u)) dst[i] = sobs[i];
       }
     }
-    if (ROLL) __syncwarp();
   }
+  if (ROLL) __syncwarp();
   }  // step loop
 
   // ---- store ----
@@ -882,6 +900,7 @@ ant_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const float*
       st.miscf[e * 2 + 1] = make_float4(T.feet[0], T.feet[1], T.feet[2], T.feet[3]);
       st.misci[e * 2 + 0] = make_int4(T.t, T.episode, T.steps_total, T.goals_left);
       st.misci[e * 2 + 1] = make_int4(T.since, T.rewarded, T.gen, 0);
+      if (ROLL && ra.ev_ret) { ra.ev_ret[e] = ev_ret; ra.ev_len[e] = ev_n < 0 ? ~ev_n : ev_n; ra.ev_fin[e] = (uint8_t)(ev_n < 0); }
     }
     if (sub == 0) st.leg[e * 4 + k] = make_float4(s.q1, s.q2, s.qd1, s.qd2);
     if (FAMILY == 0) {
@@ -1037,8 +1056,9 @@ __device__ __forceinline__ float2 mlp_policy16(const float* __restrict__ w, int 
 // 0 .. T-1 are full steps whose actions the MLP computes from the observation the previous pass left in sobs; the env
 // state stays in registers in between.  Dynamic shared memory: [EPB][64] hidden activations, then the weights.
 // ROLL = 2: ROLL = 1 with a normalized policy input (hrl_rollout_mlp_norm); mean[D] and rstd[D] follow the weights.
+// ROLL: 4 blocks per SM caps the registers at 128; left to itself ptxas picks 96 and spills the rollout's loop state
 template <int ROLL = 0>
-__global__ void __launch_bounds__(16 * HRL_POINT_EPB)
+__global__ void __launch_bounds__(16 * HRL_POINT_EPB, ROLL ? 4 : 0)
 point_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const float* __restrict__ actions,
                  const uint8_t* __restrict__ mask, float* __restrict__ obs_out_g, float* __restrict__ rew_out_g,
                  uint8_t* __restrict__ done_out_g, float* __restrict__ info_out_g, float* __restrict__ term_out_g, int mode_g,
@@ -1058,7 +1078,8 @@ point_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const floa
   if (ROLL) {
     HRL_CHECK(D <= HRL_POINT_OBS && (ra.H == 32 || ra.H == 64));
     const int nw = D * ra.H + ra.H + ra.H * ra.H + ra.H + ra.H * 2 + 2;
-    for (int i = threadIdx.x; i < nw; i += 16 * HRL_POINT_EPB) const_cast<float*>(wsm)[i] = __ldg(ra.w + i);
+    const float* wg = ra.w + (size_t)((int)blockIdx.x * HRL_POINT_EPB / ra.m_envs) * nw;   // this block's member
+    for (int i = threadIdx.x; i < nw; i += 16 * HRL_POINT_EPB) const_cast<float*>(wsm)[i] = __ldg(wg + i);
     if (ROLL == 2)
       for (int i = threadIdx.x; i < 2 * D; i += 16 * HRL_POINT_EPB) const_cast<float*>(nstat)[i] = __ldg(i < D ? ra.obs_mean + i : ra.obs_rstd + (i - D));
     __syncthreads();
@@ -1071,12 +1092,14 @@ point_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const floa
   const int n_items = cfg.n_food + cfg.n_poison, nb = cfg.n_bins;
   const bool has_item = j < n_items;
   float2 it = reinterpret_cast<const float2*>(st.items)[e * 16 + j];  // item j: food 0..n_food-1, then poison
+  float ev_ret = 0.f;  // ROLL: the launch's first episode (see ant_env_kernel)
+  int ev_n = 0;
 #pragma unroll 1
   for (int step = ROLL ? -1 : 0; step < (ROLL ? ra.T : 1); step++) {
   const int mode = ROLL ? (step < 0 ? 3 : 0) : mode_g;
-  float* __restrict__ obs_out = ROLL ? obs_out_g + (size_t)(step + 1) * N * D : obs_out_g;
-  float* __restrict__ rew_out = ROLL ? rew_out_g + (size_t)max(step, 0) * N : rew_out_g;
-  uint8_t* __restrict__ done_out = ROLL ? done_out_g + (size_t)max(step, 0) * N : done_out_g;
+  float* __restrict__ obs_out = ROLL && obs_out_g ? obs_out_g + (size_t)(step + 1) * N * D : obs_out_g;
+  float* __restrict__ rew_out = ROLL && rew_out_g ? rew_out_g + (size_t)max(step, 0) * N : rew_out_g;
+  uint8_t* __restrict__ done_out = ROLL && done_out_g ? done_out_g + (size_t)max(step, 0) * N : done_out_g;
   float* __restrict__ info_out = ROLL && info_out_g ? info_out_g + (size_t)max(step, 0) * N * 4 : info_out_g;
   float* __restrict__ term_out = ROLL && term_out_g ? term_out_g + (size_t)max(step, 0) * N * D : term_out_g;
   if (mode <= 1) {
@@ -1101,7 +1124,7 @@ point_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const floa
         sincosf(6.2831853f * u[1], &sn, &cs);
         ax += s1 * r0 * cs; ay += s2 * r0 * sn;
       }
-      if (valid && j == 0) reinterpret_cast<float2*>(ra.act_out)[(size_t)step * N + e] = make_float2(ax, ay);
+      if (valid && j == 0 && ra.act_out) reinterpret_cast<float2*>(ra.act_out)[(size_t)step * N + e] = make_float2(ax, ay);
     } else {
       ax = actions[e * 2]; ay = actions[e * 2 + 1];
     }
@@ -1197,9 +1220,10 @@ point_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const floa
       if (cfg.max_episode_steps > 0 && i0.x >= cfg.max_episode_steps) { trunc = done ? 0.f : 1.f; done = 1; }
       m0.z += food_rew;
       if (done) { m0.w += m0.z; m0.z = 0.f; }
+      if (ROLL && ev_n >= 0) { ev_ret += food_rew; ev_n = done ? ~(ev_n + 1) : ev_n + 1; }
       if (valid && j == 0) {
-        rew_out[e] = food_rew;
-        done_out[e] = (uint8_t)done;
+        if (!ROLL || rew_out) rew_out[e] = food_rew;
+        if (!ROLL || done_out) done_out[e] = (uint8_t)done;
         if (info_out) reinterpret_cast<float4*>(info_out)[e] = make_float4(food_rew, 0.f, trunc, (float)i0.x);
       }
       if (done && cfg.auto_reset) {
@@ -1220,6 +1244,7 @@ point_env_kernel(const __grid_constant__ hrl_config cfg, DevState st, const floa
       st.base[e * 4 + 2] = make_float4(vel.x, vel.y, vel.z, 0.f);
       st.miscf[e * 2 + 0] = m0;
       st.misci[e * 2 + 0] = i0;
+      if (ROLL && ra.ev_ret) { ra.ev_ret[e] = ev_ret; ra.ev_len[e] = ev_n < 0 ? ~ev_n : ev_n; ra.ev_fin[e] = (uint8_t)(ev_n < 0); }
     }
     reinterpret_cast<float2*>(st.items)[e * 16 + j] = it;
   }
@@ -1753,24 +1778,26 @@ int hrl_flagrun_next_target(hrl_handle* h, const uint8_t* d_mask, void* stream) 
 }
 
 /* Fused rollout: T env steps in ONE launch with an in-kernel MLP policy (see mlp_policy / mlp_policy16); with the
- * observation statistics, the ROLL = 2 instantiations feed the policy the normalized observation (norm_obs). */
-int hrl_rollout_mlp_norm(hrl_handle* h, int32_t T, const float* d_weights, int32_t hidden, float sigma, const float* d_sigma,
-                         uint64_t noise_seed, const float* d_obs_mean, const float* d_obs_rstd, float obs_clip, float* d_obs,
-                         float* d_act, float* d_rew, uint8_t* d_done, float* d_info, float* d_terminal_obs, void* stream) {
-  if (!h || T < 1 || !d_weights || !d_obs || !d_act || !d_rew || !d_done) return set_err(HRL_E_INVALID, "bad argument to hrl_rollout_mlp");
-  if (hidden != 32 && hidden != 64) return set_err(HRL_E_INVALID, "hrl_rollout_mlp: hidden width must be 32 or 64");
-  if (!(sigma >= 0.f)) return set_err(HRL_E_INVALID, "hrl_rollout_mlp: sigma must be >= 0");
-  if (!d_obs_mean != !d_obs_rstd)
-    return set_err(HRL_E_INVALID, "hrl_rollout_mlp_norm: d_obs_mean and d_obs_rstd must both be given or both be NULL");
+ * observation statistics, the ROLL = 2 instantiations feed the policy the normalized observation (norm_obs).  The one
+ * launch path of hrl_rollout_mlp* (P = 1, per-step buffers) and hrl_evaluate_mlp (P members, per-env results): the
+ * callers check their own buffers, the policy arguments are checked here. */
+static int launch_rollout(hrl_handle* h, const char* fn, int32_t T, int32_t P, const float* d_weights, int32_t hidden, float sigma,
+                          const float* d_sigma, uint64_t noise_seed, const float* d_obs_mean, const float* d_obs_rstd, float obs_clip,
+                          float* d_obs, float* d_act, float* d_rew, uint8_t* d_done, float* d_info, float* d_terminal_obs,
+                          float* d_ret, int32_t* d_len, uint8_t* d_finished, void* stream) {
+  if (!d_weights) return set_err(HRL_E_INVALID, fn, "d_weights is NULL");
+  if (hidden != 32 && hidden != 64) return set_err(HRL_E_INVALID, fn, "hidden width must be 32 or 64");
+  if (!(sigma >= 0.f)) return set_err(HRL_E_INVALID, fn, "sigma must be >= 0");
+  if (!d_obs_mean != !d_obs_rstd) return set_err(HRL_E_INVALID, fn, "d_obs_mean and d_obs_rstd must both be given or both be NULL");
   const bool norm = d_obs_mean != nullptr;
-  if (norm && !(obs_clip > 0.f && isfinite(obs_clip)))
-    return set_err(HRL_E_INVALID, "hrl_rollout_mlp_norm: obs_clip must be finite and > 0");
+  if (norm && !(obs_clip > 0.f && isfinite(obs_clip))) return set_err(HRL_E_INVALID, fn, "obs_clip must be finite and > 0");
   ON_DEVICE(h->device);
   DevState st = h->st;
   st.fin_flag = nullptr;
   RollArgs ra;
   ra.T = T; ra.H = hidden; ra.w = d_weights; ra.sigma = sigma; ra.sigma_v = d_sigma; ra.seed = noise_seed; ra.act_out = d_act;
   ra.obs_mean = d_obs_mean; ra.obs_rstd = d_obs_rstd; ra.obs_clip = obs_clip;
+  ra.m_envs = h->N / P; ra.ev_ret = d_ret; ra.ev_len = d_len; ra.ev_fin = d_finished;
   const int nw = h->D * hidden + hidden + hidden * hidden + hidden + hidden * h->A + h->A + (norm ? 2 * h->D : 0);
   cudaStream_t s = (cudaStream_t)stream;
   if (h->cfg.env_kind == HRL_POINT_GATHER) {
@@ -1798,6 +1825,39 @@ int hrl_rollout_mlp_norm(hrl_handle* h, int32_t T, const float* d_weights, int32
   g_launches++;
   CK(cudaGetLastError());
   return HRL_OK;
+}
+
+int hrl_rollout_mlp_norm(hrl_handle* h, int32_t T, const float* d_weights, int32_t hidden, float sigma, const float* d_sigma,
+                         uint64_t noise_seed, const float* d_obs_mean, const float* d_obs_rstd, float obs_clip, float* d_obs,
+                         float* d_act, float* d_rew, uint8_t* d_done, float* d_info, float* d_terminal_obs, void* stream) {
+  if (!h || T < 1 || !d_weights || !d_obs || !d_act || !d_rew || !d_done) return set_err(HRL_E_INVALID, "bad argument to hrl_rollout_mlp");
+  return launch_rollout(h, "hrl_rollout_mlp_norm", T, 1, d_weights, hidden, sigma, d_sigma, noise_seed, d_obs_mean, d_obs_rstd, obs_clip,
+                        d_obs, d_act, d_rew, d_done, d_info, d_terminal_obs, nullptr, nullptr, nullptr, stream);
+}
+
+int hrl_evaluate_mlp(hrl_handle* h, int32_t T, int32_t P, const float* d_weights, int32_t hidden, float sigma, const float* d_sigma,
+                     uint64_t noise_seed, const float* d_obs_mean, const float* d_obs_rstd, float obs_clip, float* d_ret,
+                     int32_t* d_len, uint8_t* d_finished, void* stream) {
+  static const char* fn = "hrl_evaluate_mlp";
+  if (!h) return set_err(HRL_E_INVALID, fn, "null handle");
+  if (T < 1) return set_err(HRL_E_INVALID, fn, "T must be >= 1");
+  if (P < 1) return set_err(HRL_E_INVALID, fn, "the member count P must be >= 1");
+  if (!d_ret || !d_len || !d_finished) return set_err(HRL_E_INVALID, fn, "d_ret, d_len and d_finished must all be given");
+  if (P > 1) {
+    // a CTA stages ONE member's weights: it must not straddle two members
+    const int epc = h->cfg.env_kind == HRL_POINT_GATHER ? HRL_POINT_EPB : Map<1>::EPW * HRL_ROLL_WARPS;
+    char msg[200];
+    if (h->N % P) {
+      snprintf(msg, sizeof msg, "num_envs %d is not a multiple of the member count %d", h->N, P);
+      return set_err(HRL_E_INVALID, fn, msg);
+    }
+    if ((h->N / P) % epc) {
+      snprintf(msg, sizeof msg, "envs per member (num_envs / P = %d) must be a multiple of %d for this env family when P > 1", h->N / P, epc);
+      return set_err(HRL_E_INVALID, fn, msg);
+    }
+  }
+  return launch_rollout(h, fn, T, P, d_weights, hidden, sigma, d_sigma, noise_seed, d_obs_mean, d_obs_rstd, obs_clip, nullptr, nullptr,
+                        nullptr, nullptr, nullptr, nullptr, d_ret, d_len, d_finished, stream);
 }
 
 int hrl_rollout_mlp_ex(hrl_handle* h, int32_t T, const float* d_weights, int32_t hidden, float sigma, const float* d_sigma,

@@ -321,11 +321,44 @@ class VecEnv:
     @staticmethod
     def pack_mlp(layers):
         """Pack ((W1, b1), (W2, b2), (W3, b3)) in torch.nn.Linear layout (W[out, in]) into the input-major float32 vector
-        `hrl_rollout_mlp` reads: W1^T b1 W2^T b2 W3^T b3."""
+        `hrl_rollout_mlp` reads: W1^T b1 W2^T b2 W3^T b3.  Batched layers (W[P, out, in], b[P, out]: one policy per member
+        of a population) pack into [P, nw], one such vector per row (`hrl_evaluate_mlp`)."""
         parts = []
         for W, b in layers:
-            parts += [W.detach().to(torch.float32).t().contiguous().reshape(-1), b.detach().to(torch.float32).reshape(-1)]
-        return torch.cat(parts).contiguous()
+            W, b = W.detach().to(torch.float32), b.detach().to(torch.float32)
+            if W.dim() == 3:
+                parts += [W.transpose(1, 2).reshape(W.shape[0], -1), b.reshape(b.shape[0], -1)]
+            else:
+                parts += [W.t().contiguous().reshape(-1), b.reshape(-1)]
+        return torch.cat(parts, dim=-1).contiguous()
+
+    def _mlp_width(self, layers, batched=False):
+        """Hidden width H of ((W1[H, D], b1[H]), (W2[H, H], b2[H]), (W3[A, H], b3[A])), with a leading member dimension P
+        on every tensor when `batched`; returns (H, P) (P = None unbatched).  ValueError on any other shape."""
+        (W1, b1), (W2, b2), (W3, b3) = layers
+        lead = tuple(W1.shape[:1]) if batched else ()
+        H = W1.shape[len(lead)] if W1.dim() == len(lead) + 2 else -1
+        want = ((H, self.D), (H,), (H, H), (H,), (self.A, H), (self.A,))
+        if H not in (32, 64) or (batched and lead[0] < 1) or any(tuple(t.shape) != lead + s for t, s in zip((W1, b1, W2, b2, W3, b3), want)):
+            p = "P," if batched else ""
+            raise ValueError("layers must be ((W1[{p}H,{D}], b1[{p}H]), (W2[{p}H,H], b2[{p}H]), (W3[{p}{A},H], b3[{p}{A}])) with H = 32 or 64, "
+                             "got W1 of shape {s}".format(p=p, D=self.D, A=self.A, s=tuple(W1.shape)))
+        return H, (lead[0] if batched else None)
+
+    def _noise_scale(self, sigma):
+        """(scalar sigma, per-component scale tensor or None) for the C-ABI, from a float or a length-A tensor."""
+        if not isinstance(sigma, torch.Tensor):
+            return sigma, None
+        sig_v = sigma.detach().to(device=self.device, dtype=torch.float32).contiguous()
+        if tuple(sig_v.shape) != (self.A,):
+            raise ValueError("sigma must be a float or a tensor of %d entries, got shape %s" % (self.A, tuple(sig_v.shape)))
+        if not bool((torch.isfinite(sig_v) & (sig_v >= 0)).all()):
+            raise ValueError("sigma entries must be finite and >= 0")
+        return 0.0, sig_v
+
+    def _check_obs_norm(self, obs_norm):
+        if obs_norm is not None and (getattr(obs_norm, "D", None) != self.D or getattr(obs_norm, "device", None) != self.device):
+            raise ValueError("obs_norm must be a RunningNormalizer of obs_dim %d on %s" % (self.D, self.device))
 
     def rollout_mlp(self, layers, horizon, buf=None, sigma=0.0, noise_seed=0, want_info=False, want_terminal_obs=False,
                     obs_norm=None):
@@ -341,16 +374,8 @@ class VecEnv:
         if H not in (32, 64) or tuple(W1.shape) != (H, self.D) or tuple(W2.shape) != (H, H) or tuple(W3.shape) != (self.A, H):
             raise ValueError("layers must be ((W1[H,%d], b1[H]), (W2[H,H], b2[H]), (W3[%d,H], b3[%d])) with H = 32 or 64" % (self.D, self.A, self.A))
         w = self.pack_mlp(layers).to(self.device)
-        sig_v = None
-        if isinstance(sigma, torch.Tensor):
-            sig_v = sigma.detach().to(device=self.device, dtype=torch.float32).contiguous()
-            if tuple(sig_v.shape) != (self.A,):
-                raise ValueError("sigma must be a float or a tensor of %d entries, got shape %s" % (self.A, tuple(sig_v.shape)))
-            if not bool((torch.isfinite(sig_v) & (sig_v >= 0)).all()):
-                raise ValueError("sigma entries must be finite and >= 0")
-            sigma = 0.0
-        if obs_norm is not None and (getattr(obs_norm, "D", None) != self.D or getattr(obs_norm, "device", None) != self.device):
-            raise ValueError("obs_norm must be a RunningNormalizer of obs_dim %d on %s" % (self.D, self.device))
+        sigma, sig_v = self._noise_scale(sigma)
+        self._check_obs_norm(obs_norm)
         buf = buf or RolloutBuffer(self, horizon, info=want_info, terminal_obs=want_terminal_obs)
         if buf.T < horizon:
             raise ValueError("rollout buffer holds %d steps, need %d" % (buf.T, horizon))
@@ -373,6 +398,57 @@ class VecEnv:
             torch.cuda.nvtx.range_pop()
         self._keep = (w, sig_v)   # the launch is asynchronous: keep the packed weights and noise scales alive
         return buf
+
+    def evaluate_mlp(self, layers, horizon, sigma=0.0, noise_seed=0, obs_norm=None, out=None):
+        """Score MLP policies by their episodes in ONE kernel launch (include/hrl_b200.h `hrl_evaluate_mlp`), writing no
+        per-step buffers.  `layers`: the layers of `rollout_mlp` (one policy for all envs, P = 1) or batched, every tensor
+        with a leading member dimension P (W1[P, H, D], b1[P, H], ...).  Env e runs member e // M, M = N / P; for P > 1, N
+        must be a multiple of P and M a multiple of 16 (Ant) or 8 (PointGather).  `sigma`, `noise_seed` and `obs_norm` act as
+        in `rollout_mlp`, the same for every member.
+        Runs `horizon` steps from the current state, with auto-reset.  Returns `(ret, length, finished)`, [P, M] views of [N]
+        tensors (row m: member m's envs): the float32 sum of each env's rewards from the first step up to and including its
+        first done, the number of those steps, and whether a done came within `horizon` steps (if not, the sum covers all of
+        them).  Call `reset()` first to score whole episodes: an env started mid-episode is scored on the rest of it.
+        `out=(ret f32, length i32, finished bool)`, each [N] or [P, M]: written in place (no allocation, so the call can be
+        captured in a CUDA graph).  No host synchronisation, except to check a sigma tensor's entries."""
+        H, P = self._mlp_width(layers, batched=layers[0][0].dim() == 3)
+        P = P or 1
+        T = int(horizon)
+        if T < 1:
+            raise ValueError("horizon must be >= 1, got %d" % T)
+        epc = 8 if self.kind == HRL_POINT_GATHER else 16
+        if self.N % P:
+            raise ValueError("num_envs %d is not a multiple of the member count %d" % (self.N, P))
+        M = self.N // P
+        if P > 1 and M % epc:
+            raise ValueError("envs per member (num_envs / P = %d) must be a multiple of %d for %s" % (M, epc, self.env_id))
+        sigma, sig_v = self._noise_scale(sigma)
+        if sig_v is None and not float(sigma) >= 0.0:
+            raise ValueError("sigma must be >= 0, got %r" % (sigma,))
+        self._check_obs_norm(obs_norm)
+        if out is None:
+            ret = torch.empty(self.N, device=self.device)
+            length = torch.empty(self.N, dtype=torch.int32, device=self.device)
+            finished = torch.empty(self.N, dtype=torch.bool, device=self.device)
+        else:
+            if len(out) != 3:
+                raise ValueError("out must be (ret, length, finished)")
+            ret, length, finished = out
+            for t, dt in ((ret, torch.float32), (length, torch.int32), (finished, torch.bool)):
+                if not isinstance(t, torch.Tensor) or tuple(t.shape) not in ((self.N,), (P, M)) or t.dtype != dt or not t.is_contiguous() \
+                        or t.device != self.device:
+                    raise ValueError("out must be contiguous tensors on %s of shape [%d] or [%d, %d]: ret float32, length int32, finished "
+                                     "bool" % (self.device, self.N, P, M))
+        w = self.pack_mlp(layers).to(self.device)
+        if _NVTX:
+            torch.cuda.nvtx.range_push("hrl.evaluate_mlp")
+        norm = (None, None, 0.0) if obs_norm is None else (obs_norm.mean, obs_norm.rstd, obs_norm.clip_obs)
+        _cabi.check(self.L.hrl_evaluate_mlp(self.h, T, P, _ptr(w), int(H), float(sigma), _ptr(sig_v), int(noise_seed), _ptr(norm[0]),
+                                            _ptr(norm[1]), float(norm[2]), _ptr(ret), _ptr(length), _ptr(finished), self._stream()))
+        if _NVTX:
+            torch.cuda.nvtx.range_pop()
+        self._keep = (w, sig_v)   # the launch is asynchronous: keep the packed weights and noise scales alive
+        return ret.view(P, M), length.view(P, M), finished.view(P, M)
 
     def rollout_buffer(self, horizon):
         """Device-resident storage for ``horizon`` steps; ``step(a, out=buf.slot(t))`` fills slot t in place."""

@@ -241,6 +241,27 @@ int hrl_rollout_mlp_norm(hrl_handle* h, int32_t T, const float* d_weights, int32
                          float* d_obs, float* d_act, float* d_rew, uint8_t* d_done, float* d_info, float* d_terminal_obs,
                          void* stream);
 
+/* Score a population of P MLP policies by their episodes, in ONE launch and without per-step buffers (evolution
+ * strategies, population-based training, comparing checkpoints).  The policy, noise and auto-reset are those of
+ * hrl_rollout_mlp_norm; what differs is that each env runs its member's weights and that only per-env results are written.
+ *   d_weights  f32[P][nw]: P rows in the packed layout of hrl_rollout_mlp, nw = D*H + H + H*H + H + H*A + A.
+ *   Env e runs member e / M, M = N / P.  P = 1: any N.  P > 1: N must be a multiple of P and M a multiple of the envs
+ *   one CTA runs, 16 for the Ant families and 8 for PointGather (a CTA stages one member's weights); otherwise
+ *   HRL_E_INVALID.
+ *   sigma, d_sigma, noise_seed, d_obs_mean, d_obs_rstd, obs_clip: as in hrl_rollout_mlp_norm, shared by every member (the
+ *   same noise draw for the same seed, global env index and step count; the statistics frozen for the launch).
+ * T steps run from the current state; nothing per step is written.  Per env:
+ *   d_ret      f32[N]: the sum of the rewards from the launch's first step up to and including the env's first done,
+ *              accumulated in float32 in step order (ret += rew);
+ *   d_len      i32[N]: the number of those steps;
+ *   d_finished u8[N]:  1 if a done came within the T steps; else 0, and d_ret / d_len cover all T steps.
+ * The env state afterwards is the state after T steps, the one hrl_rollout_mlp would leave.  To score whole episodes, reset
+ * first (hrl_reset): a launch that starts mid-episode scores the remainder of that episode.  T >= 1, P >= 1, hidden = 32 or
+ * 64, and the three result pointers are required. */
+int hrl_evaluate_mlp(hrl_handle* h, int32_t T, int32_t P, const float* d_weights, int32_t hidden, float sigma, const float* d_sigma,
+                     uint64_t noise_seed, const float* d_obs_mean, const float* d_obs_rstd, float obs_clip, float* d_ret,
+                     int32_t* d_len, uint8_t* d_finished, void* stream);
+
 /* Replaces saveState/restoreState (used as the reset mechanism by pybullet_envs) and gives
  * the "identical saved states" hook the one-step parity tests need.
  *   d_fstate f32[N, HRL_STATE_F], d_istate i32[N, HRL_STATE_I]. */
